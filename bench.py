@@ -9,6 +9,7 @@ are the only thing that scales, SURVEY.md section 8(e)).  Work model is the refe
 TFLOP/s counts the two GEMMs only, 4*N^2*D per head.
 
     python bench.py --gpus 1 --steps 50 --warmup 5            # our arm
+    python bench.py --gpus 1 --steps 50 --warmup 5 --dump-outputs DIR   # ... and keep a sample of O and L to compare
     python bench.py --impl reference --gpus 1 --steps 3 --warmup 1   # the reference's CPU path (oracle port)
     python -m torch.distributed.run --nproc-per-node N ... bench.py --gpus N ...
 
@@ -45,6 +46,21 @@ UNIT = "GINSTRS"
 # (profiles/), for the default H; None until a capture exists.
 NCU_TRAFFIC_BYTES_PER_LAUNCH = 298728960  # profiles/r2_fwd_ncu_summary.csv: 201.77 MB read + 96.96 MB written
 NCU_TRAFFIC_SOURCE = "profiles/r2_fwd_ncu_summary.csv (ncu --set full, one 64-head launch of this kernel; not re-measured in this run)"
+# --dump-outputs keeps this many (head, row) rows of O and L: 32 MiB of O at D=128, whatever --heads is
+DUMP_ROWS, DUMP_SEED = 65536, 0
+
+
+def dump_outputs(directory, o, lse):
+    """Write a fixed, seeded sample of the rows of O [H, N, D] and L [H, N] as float32 .npy files.  The sample depends
+    only on H and N, so two builds run with the same arguments can be compared output for output."""
+    import numpy as np
+    import torch
+    rows = o.shape[0] * o.shape[1]
+    pick = np.sort(np.random.default_rng(DUMP_SEED).choice(rows, size=min(rows, DUMP_ROWS), replace=False))
+    index = torch.from_numpy(pick).to(o.device)
+    os.makedirs(directory, exist_ok=True)
+    np.save(os.path.join(directory, "O.npy"), o.reshape(rows, -1).index_select(0, index).float().cpu().numpy())
+    np.save(os.path.join(directory, "L.npy"), lse.reshape(rows).index_select(0, index).float().cpu().numpy())
 
 
 def measured_peaks():
@@ -288,7 +304,12 @@ def main():
     ap.add_argument("--no-sustained", action="store_true")
     ap.add_argument("--sustained-seconds", type=float, default=2.0)
     ap.add_argument("--config5-heads", type=int, default=2048, help="batch 64 x heads 32 of BASELINE.json configs[4]")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed steps, write rank 0's O and L of the last timed step to DIR/O.npy and DIR/L.npy "
+                         f"(float32; a fixed seeded sample of at most {DUMP_ROWS} of the heads x N rows)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     args.warmup = max(args.warmup, 3) if args.impl == "ours" else args.warmup
 
     rank = int(os.environ.get("RANK", "0"))
@@ -374,6 +395,9 @@ def main():
     total_heads = H * world
     value = FMA_PER_HEAD * total_heads / (ms_per_step * 1e-3) / 1e9
     tflops = FLOP_PER_HEAD * total_heads / (ms_per_step * 1e-3) / 1e12
+    if args.dump_outputs and rank == 0:   # before the legs below launch on the same buffers again
+        last = sets[(args.steps - 1) & 1]
+        dump_outputs(args.dump_outputs, last[Op.O], last[Op.L])
 
     # ---- `e2e`: host buffers through mfa_attention_run_host ------------------------------------
     e2e = None
