@@ -14,11 +14,33 @@
 
 #include "internal.h"
 #include "kernels/device_state.h"
+#include "kernels/tma_host.h"
+
+namespace mfa {
+// The tcgen05 kernel that serves a descriptor; decided once, when the kernel object is created.
+enum class Tcgen05Family : uint8_t {
+  kForward,           // row-major, pad8(D) <= 128 (tcgen05_forward.cu)
+  kForwardWide,       // row-major, 128 < pad8(D) <= 256 (tcgen05_forward_d256.cu)
+  kForwardGeneric,    // transposed operands (tcgen05_forward_d256.cu)
+  kBackward,          // row-major, pad8(D) <= 128 (tcgen05_backward.cu)
+  kBackwardGeneric,   // transposed operands, or pad8(D) > 128 (tcgen05_backward_generic.cu)
+};
+
+// `transposed`: any of the operands the launchers look at is transposed -- Q, K, V, O for the forward, all eight matrix
+// operands for the backward kernels
+static Tcgen05Family tcgen05_family(int type, uint32_t padded_head, bool transposed) {
+  if (type == MFA_FORWARD)
+    return transposed ? Tcgen05Family::kForwardGeneric
+                      : (padded_head > 128 ? Tcgen05Family::kForwardWide : Tcgen05Family::kForward);
+  return transposed || padded_head > 128 ? Tcgen05Family::kBackwardGeneric : Tcgen05Family::kBackward;
+}
+}  // namespace mfa
 
 struct mfa_attention_kernel {
   mfa_attention_kernel_descriptor_t descriptor;
   int type;
   int backend;
+  mfa::Tcgen05Family family;  // (backend == MFA_BACKEND_TCGEN05 only)
   uint32_t threads, smem_bytes, par, trav, head;
   std::string source_name;
 };
@@ -99,6 +121,28 @@ static int build_params(const mfa_attention_kernel *k, const mfa_function_consta
   return MFA_SUCCESS;
 }
 
+// The encode-time checks (R and C against the TMA pitch rule for transposed operands, output precisions) come after the
+// head-dimension padding copies have been queued, then the kernel chosen at creation is launched.
+static cudaError_t launch_tcgen05(const mfa_attention_kernel *k, const AttentionParams &p, cudaStream_t stream) {
+  const bool key_value = k->type == MFA_BACKWARD_KEY_VALUE;
+  if (k->type == MFA_FORWARD && !tcgen05_forward_supported(p)) {
+    set_launch_detail("descriptor is outside the tcgen05 forward kernel's domain");
+    return cudaErrorInvalidValue;
+  }
+  if (k->type != MFA_FORWARD && !tcgen05_backward_supported(p)) {
+    set_launch_detail("descriptor is outside the tcgen05 backward kernels' domain");
+    return cudaErrorInvalidValue;
+  }
+  switch (k->family) {
+    case Tcgen05Family::kForward: return launch_tcgen05_forward(p, stream);
+    case Tcgen05Family::kForwardWide: return launch_tcgen05_forward_d256(p, stream);
+    case Tcgen05Family::kForwardGeneric: return launch_tcgen05_forward_generic(p, stream);
+    case Tcgen05Family::kBackward: return launch_tcgen05_backward(p, stream, key_value);
+    case Tcgen05Family::kBackwardGeneric: return launch_tcgen05_backward_generic(p, stream, key_value);
+  }
+  return cudaErrorInvalidValue;
+}
+
 }  // namespace mfa
 
 using namespace mfa;
@@ -165,14 +209,25 @@ int mfa_attention_kernel_create(const mfa_attention_kernel_descriptor_t *kd, mfa
                                              "/4 has no compiled sm_100a kernel (available: 0.." +
                                              std::to_string(max_quarters) + ").");
     }
-    if (k->type == MFA_FORWARD && transposed)
-      tcgen05_forward_generic_geometry(D, &k->threads, &k->smem_bytes, &k->par, &k->trav, &k->head);
-    else if (k->type == MFA_FORWARD)
-      tcgen05_forward_geometry(Dp, &k->threads, &k->smem_bytes, &k->par, &k->trav, &k->head);
-    else if (transposed || Dp > 128)
-      tcgen05_backward_generic_geometry(k->type, Dp, &k->threads, &k->smem_bytes, &k->par, &k->trav, &k->head);
-    else
-      tcgen05_backward_geometry(k->type, Dp, &k->threads, &k->smem_bytes, &k->par, &k->trav, &k->head);
+    constexpr uint16_t kForwardMatrices = (1u << MFA_Q) | (1u << MFA_K) | (1u << MFA_V) | (1u << MFA_O);
+    constexpr uint16_t kAllMatrices = kForwardMatrices | (1u << MFA_dO) | (1u << MFA_dV) | (1u << MFA_dK) | (1u << MFA_dQ);
+    const uint16_t routed = k->type == MFA_FORWARD ? kForwardMatrices : kAllMatrices;
+    k->family = tcgen05_family(k->type, Dp, (kd->transpose_state_mask & routed) != 0);
+    switch (k->family) {
+      case Tcgen05Family::kForward:
+        tcgen05_forward_geometry(Dp, &k->threads, &k->smem_bytes, &k->par, &k->trav, &k->head);
+        break;
+      case Tcgen05Family::kForwardWide:
+      case Tcgen05Family::kForwardGeneric:
+        tcgen05_forward_generic_geometry(Dp, &k->threads, &k->smem_bytes, &k->par, &k->trav, &k->head);
+        break;
+      case Tcgen05Family::kBackward:
+        tcgen05_backward_geometry(k->type, Dp, &k->threads, &k->smem_bytes, &k->par, &k->trav, &k->head);
+        break;
+      case Tcgen05Family::kBackwardGeneric:
+        tcgen05_backward_generic_geometry(k->type, Dp, &k->threads, &k->smem_bytes, &k->par, &k->trav, &k->head);
+        break;
+    }
   } else if (k->backend == MFA_BACKEND_SIMT_FP32) {
     if (D > 512) {
       delete k;
@@ -193,9 +248,12 @@ int mfa_attention_kernel_create(const mfa_attention_kernel_descriptor_t *kd, mfa
     return fail(MFA_ERROR_UNSUPPORTED, msg);
   }
   static const char *typeNames[] = {"forward", "backward_query", "backward_key_value"};
+  // the exp2 column selects an instantiation of the D <= 128 row-major kernels only
+  const bool exp2_variants = k->backend == MFA_BACKEND_TCGEN05 &&
+                             (k->family == Tcgen05Family::kForward || k->family == Tcgen05Family::kBackward);
   k->source_name = std::string("attention_") + typeNames[k->type] +
                    (k->backend == MFA_BACKEND_TCGEN05 ? "_tcgen05" : "_simt_fp32") + "<D=" + std::to_string(D) +
-                   (k->backend == MFA_BACKEND_TCGEN05 && k->trav == 128 && D <= 128 && kd->exp2_fma_quarters
+                   (exp2_variants && kd->exp2_fma_quarters
                         ? ", exp2 on FMA pipe " + std::to_string(kd->exp2_fma_quarters) + "/4"
                         : std::string()) +
                    ">";
@@ -244,26 +302,28 @@ int mfa_attention_kernel_launch_count(const mfa_attention_kernel_t *kernel, cons
                                       uint32_t *out) {
   if (!kernel || !c || !out) return fail(MFA_ERROR_INVALID_ARGUMENT, "NULL argument.");
   *out = 1;
-  const uint16_t forward_operands = (1u << MFA_Q) | (1u << MFA_K) | (1u << MFA_V) | (1u << MFA_O);
-  if (kernel->backend == MFA_BACKEND_TCGEN05 && kernel->type == MFA_FORWARD &&
-      !(kernel->descriptor.transpose_state_mask & forward_operands))  // (the layout-generic kernel never splits)
-    *out = tcgen05_forward_launch_count(c->row, c->column, kernel->descriptor.head_dimension,
-                                        c->batch_count ? c->batch_count : 1, kernel->descriptor.split_min_blocks,
-                                        kernel->descriptor.split_max);
-  if (kernel->backend == MFA_BACKEND_TCGEN05 && kernel->type != MFA_FORWARD) {
-    const uint16_t any = kernel->descriptor.transpose_state_mask & kernel->descriptor.transpose_state_valid_mask;
-    const uint32_t Dp = (kernel->descriptor.head_dimension + 7u) / 8u * 8u;
-    const uint32_t b = c->batch_count ? c->batch_count : 1;
-    const bool convert = kernel->descriptor.memory_precisions[MFA_dO] != kernel->descriptor.memory_precisions[MFA_Q];
-    *out = (any || Dp > 128)
-               ? tcgen05_backward_generic_launch_count(kernel->type, c->row, c->column, Dp, b, kernel->descriptor.split_min_blocks,
-                                                       kernel->descriptor.split_max, convert)
-               : tcgen05_backward_launch_count(kernel->type, c->row, c->column, b, kernel->descriptor.split_min_blocks,
-                                               kernel->descriptor.split_max, convert);
+  if (kernel->backend != MFA_BACKEND_TCGEN05) return MFA_SUCCESS;
+  const mfa_attention_kernel_descriptor_t &kd = kernel->descriptor;
+  const uint32_t Dp = (kd.head_dimension + 7u) / 8u * 8u;
+  const uint32_t b = c->batch_count ? c->batch_count : 1;
+  const bool convert = kd.memory_precisions[MFA_dO] != kd.memory_precisions[MFA_Q];
+  switch (kernel->family) {
+    case Tcgen05Family::kForward:
+      *out = tcgen05_forward_launch_count(c->row, c->column, b, kd.split_min_blocks, kd.split_max);
+      break;
+    case Tcgen05Family::kForwardWide:
+    case Tcgen05Family::kForwardGeneric:
+      break;  // (these never split)
+    case Tcgen05Family::kBackward:
+      *out = tcgen05_backward_launch_count(kernel->type, c->row, c->column, b, kd.split_min_blocks, kd.split_max, convert);
+      break;
+    case Tcgen05Family::kBackwardGeneric:
+      *out = tcgen05_backward_generic_launch_count(kernel->type, c->row, c->column, Dp, b, kd.split_min_blocks, kd.split_max,
+                                                   convert);
+      break;
   }
-  // head % 8 != 0 on the tensor-core family: one padding copy per staged input, one un-padding copy per output
-  if (kernel->backend == MFA_BACKEND_TCGEN05 && kernel->descriptor.head_dimension % 8 != 0)
-    *out += kernel->type == MFA_FORWARD ? 4 : (kernel->type == MFA_BACKWARD_QUERY ? 6 : 6);
+  // head % 8 != 0: one padding copy per staged input, one un-padding copy per output
+  if (kd.head_dimension % 8 != 0) *out += kernel->type == MFA_FORWARD ? 4 : 6;
   return MFA_SUCCESS;
 }
 
@@ -321,7 +381,7 @@ int mfa_attention_kernel_encode(const mfa_attention_kernel_t *kernel, const mfa_
       void *ws = nullptr;
       if ((e = workspace_for(device, stream, total, &ws, /*slot=*/1)) != cudaSuccess)
         return fail(MFA_ERROR_CUDA, std::string("padding workspace: ") + cudaGetErrorString(e) + " " + last_launch_detail());
-      char *cursor = static_cast<char *>(ws) + kWorkspaceCounterBytes;
+      char *cursor = static_cast<char *>(ws);
       for (int i = 0; i < nin && e == cudaSuccess; ++i) {
         const int slot = ins[i];
         e = launch_pad_columns(q.buf[slot], cursor, rows_of(slot), p.D, Dp, p.prec[slot] == FP32 ? 4 : 2, stream);
@@ -339,11 +399,7 @@ int mfa_attention_kernel_encode(const mfa_attention_kernel_t *kernel, const mfa_
         return fail(MFA_ERROR_CUDA, std::string("head-dimension padding failed: ") + cudaGetErrorString(e));
     }
     if (kernel->backend == MFA_BACKEND_TCGEN05) {
-      switch (kernel->type) {
-        case MFA_FORWARD: e = launch_tcgen05_forward(q, stream); break;
-        case MFA_BACKWARD_QUERY: e = launch_tcgen05_backward_query(q, stream); break;
-        default: e = launch_tcgen05_backward_key_value(q, stream); break;
-      }
+      e = launch_tcgen05(kernel, q, stream);
     } else {
       switch (kernel->type) {
         case MFA_FORWARD: e = launch_simt_forward(q, stream); break;
@@ -371,17 +427,19 @@ int mfa_attention_kernel_encode(const mfa_attention_kernel_t *kernel, const mfa_
 MFA_API int mfa_debug_forward_trace(const mfa_attention_kernel_t *kernel, const mfa_function_constants_t *constants,
                                     void *const buffers[MFA_BUFFER_COUNT], void *cuda_stream, long long *trace) {
   if (!kernel || !constants || !buffers || !trace) return fail(MFA_ERROR_INVALID_ARGUMENT, "NULL argument.");
+  const bool row_major_forward = kernel->backend == MFA_BACKEND_TCGEN05 && (kernel->family == Tcgen05Family::kForward ||
+                                                                           kernel->family == Tcgen05Family::kForwardWide);
+  if (!row_major_forward)
+    return fail(MFA_ERROR_INVALID_ARGUMENT, "Pipeline traces exist for the row-major tcgen05 forward kernels only.");
   AttentionParams p;
   int status = build_params(kernel, constants, buffers, p);
   if (status != MFA_SUCCESS) return status;
-  cudaError_t e = p.D > 128 ? launch_tcgen05_forward_d256_trace(p, static_cast<cudaStream_t>(cuda_stream), trace)
-                            : launch_tcgen05_forward_trace(p, static_cast<cudaStream_t>(cuda_stream), trace);
+  cudaStream_t stream = static_cast<cudaStream_t>(cuda_stream);
+  cudaError_t e = kernel->family == Tcgen05Family::kForwardWide ? launch_tcgen05_forward_d256_trace(p, stream, trace)
+                                                                : launch_tcgen05_forward_trace(p, stream, trace);
   if (e != cudaSuccess) return fail(MFA_ERROR_CUDA, std::string("trace launch failed: ") + cudaGetErrorString(e));
   return MFA_SUCCESS;
 }
-
-// Debug-only export: 0 forces split-KV onto its scratch + combine fallback (tests cover both forms).
-MFA_API void mfa_debug_set_forward_fused(int enabled) { tcgen05_forward_set_fused(enabled); }
 
 // ------------------------------------------------------------------------------------------------
 // Kernel cache keyed by descriptor -- the useful half of the reference's pipeline cache

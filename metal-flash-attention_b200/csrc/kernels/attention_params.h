@@ -39,23 +39,23 @@ cudaError_t launch_simt_backward_key_value(const AttentionParams &p, cudaStream_
 void simt_geometry(int type, uint32_t D, uint32_t *threads, uint32_t *smem_bytes, uint32_t *par, uint32_t *trav,
                    uint32_t *head);
 
-// ---- tcgen05 / TMA / TMEM family (16-bit row-major inputs, D % 8 == 0) ----------------------
-struct Tcgen05Plan;  // owns tensor maps; defined in tcgen05_common.h
+// ---- tcgen05 / TMA / TMEM family (16-bit inputs, D % 8 == 0) --------------------------------
+// kernel.cpp picks the kernel of a descriptor once, at creation; each launcher below serves only its own kernel.
+// The *_supported checks validate the encode-time R, C and output precisions against what these kernels handle.
 bool tcgen05_forward_supported(const AttentionParams &p);
-cudaError_t launch_tcgen05_forward(const AttentionParams &p, cudaStream_t stream);
+cudaError_t launch_tcgen05_forward(const AttentionParams &p, cudaStream_t stream);  // row-major, D <= 128
 void tcgen05_forward_geometry(uint32_t D, uint32_t *threads, uint32_t *smem_bytes, uint32_t *par, uint32_t *trav,
                               uint32_t *head);
-uint32_t tcgen05_forward_launch_count(uint32_t R, uint32_t C, uint32_t D, uint32_t batch, uint32_t min_blocks,
-                                      uint32_t max_splits);
-cudaError_t launch_tcgen05_forward_d256(const AttentionParams &p, cudaStream_t stream);  // 128 < D <= 256
+uint32_t tcgen05_forward_launch_count(uint32_t R, uint32_t C, uint32_t batch, uint32_t min_blocks, uint32_t max_splits);
+cudaError_t launch_tcgen05_forward_d256(const AttentionParams &p, cudaStream_t stream);  // row-major, 128 < D <= 256
 cudaError_t launch_tcgen05_forward_generic(const AttentionParams &p, cudaStream_t stream);  // transposed operands, D <= 256
 bool tcgen05_forward_transposes_ok(uint32_t R, uint32_t C, bool tQ, bool tK, bool tV);
+// geometry of the kernel template behind both launch_tcgen05_forward_d256 and launch_tcgen05_forward_generic
 void tcgen05_forward_generic_geometry(uint32_t D, uint32_t *threads, uint32_t *smem_bytes, uint32_t *par, uint32_t *trav,
                                       uint32_t *head);
-void tcgen05_forward_d256_geometry(uint32_t *threads, uint32_t *smem_bytes, uint32_t *par, uint32_t *trav);
 bool tcgen05_backward_supported(const AttentionParams &p);
-cudaError_t launch_tcgen05_backward_query(const AttentionParams &p, cudaStream_t stream);
-cudaError_t launch_tcgen05_backward_key_value(const AttentionParams &p, cudaStream_t stream);
+// row-major, D <= 128; key_value: dK and dV, else dQ (and the D term)
+cudaError_t launch_tcgen05_backward(const AttentionParams &p, cudaStream_t stream, bool key_value);
 uint32_t tcgen05_backward_launch_count(int type, uint32_t R, uint32_t C, uint32_t batch, uint32_t min_blocks,
                                        uint32_t max_splits, bool convert_dO);
 bool tcgen05_backward_converts_dO_first(uint32_t C, uint32_t batch);
@@ -69,7 +69,6 @@ uint32_t tcgen05_backward_generic_launch_count(int type, uint32_t R, uint32_t C,
 void tcgen05_backward_generic_geometry(int type, uint32_t D, uint32_t *threads, uint32_t *smem_bytes, uint32_t *par,
                                        uint32_t *trav, uint32_t *head);
 
-void tcgen05_forward_set_fused(int enabled);  // debug: 0 = split-KV through scratch + combine kernel (two launches)
 cudaError_t launch_tcgen05_forward_trace(const AttentionParams &p, cudaStream_t stream, long long *trace);  // debug
 cudaError_t launch_tcgen05_forward_d256_trace(const AttentionParams &p, cudaStream_t stream, long long *trace);  // debug
 // head-dimension padding for D % 8 != 0 on the tensor-core family (pad_head.cu)

@@ -61,14 +61,13 @@ std::map<std::pair<std::pair<int, int>, cudaStream_t>, Workspace> g_workspaces; 
 cudaError_t workspace_for(int device, cudaStream_t stream, size_t bytes, void **out, int slot) {
   std::lock_guard<std::mutex> lock(g_workspace_mutex);
   Workspace &w = g_workspaces[std::make_pair(std::make_pair(device, slot), stream)];
-  const size_t need = bytes + kWorkspaceCounterBytes;
-  if (w.bytes < need) {
+  if (w.bytes < bytes) {
     // growing means allocating: not possible while the stream is being captured into a graph (warm the kernel up once
     // before capturing, as every graph user does)
     cudaStreamCaptureStatus capture = cudaStreamCaptureStatusNone;
     if (cudaStreamIsCapturing(stream, &capture) == cudaSuccess && capture != cudaStreamCaptureStatusNone) {
       set_launch_detail("the split-grid workspace (%zu bytes) must be allocated before stream capture: run the kernel "
-                        "once outside the capture first", need);
+                        "once outside the capture first", bytes);
       return cudaErrorStreamCaptureUnsupported;
     }
     if (w.ptr) {
@@ -79,13 +78,12 @@ cudaError_t workspace_for(int device, cudaStream_t stream, size_t bytes, void **
       w.ptr = nullptr;
       w.bytes = 0;
     }
-    size_t rounded = (need + (size_t(1) << 20) - 1) & ~((size_t(1) << 20) - 1);
+    size_t rounded = (bytes + (size_t(1) << 20) - 1) & ~((size_t(1) << 20) - 1);
     cudaError_t e = cudaMalloc(&w.ptr, rounded);
     if (e != cudaSuccess) {
       set_launch_detail("cudaMalloc of the %zu-byte split-grid workspace failed", rounded);
       return e;
     }
-    if ((e = cudaMemsetAsync(w.ptr, 0, kWorkspaceCounterBytes, stream)) != cudaSuccess) return e;
     w.bytes = rounded;
   }
   *out = w.ptr;

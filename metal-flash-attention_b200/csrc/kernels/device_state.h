@@ -23,11 +23,10 @@ cudaError_t ensure_max_dynamic_smem(const void *kernel, uint32_t bytes, int devi
 // Library-owned scratch for kernels that split small grids (forward split-KV partials, backward traversal splits): one
 // growing allocation per (device, stream), so launches on one stream reuse it in stream order and launches on
 // different streams never share it.  `*out` stays valid until the next request for the same (device, stream) that
-// needs more room.  The first `kWorkspaceCounterBytes` bytes of every workspace are arrival counters, zeroed at
-// allocation and returned to zero by the kernels that use them.
-constexpr size_t kWorkspaceCounterBytes = 4096;
+// needs more room.  The block is cudaMalloc-aligned (256 B), which the tensor map over the forward's split partials needs.
 // `slot` separates independent users inside one encode(): 0 = split partials (forward / backward launchers), 1 = the
-// head-dimension padding staging of kernel.cpp, which is live across the launcher's own use of slot 0.
+// head-dimension padding staging of kernel.cpp, which is live across the launcher's own use of slot 0, 2 = the FP16
+// copy of a BF16 dO (backward launchers), which is live across their use of slot 0.
 cudaError_t workspace_for(int device, cudaStream_t stream, size_t bytes, void **out, int slot = 0);
 
 // Frees every workspace of `device` (the device must be idle); used by tests and by mfa_release_device_resources().

@@ -364,26 +364,16 @@ __device__ __forceinline__ float2 unpack_f16x2(uint32_t w) {
 }
 
 // ---------------------------------------------------------------- online-softmax inner loop ---
-// l accumulates the P values the tensor core will actually multiply (rounded to the 16-bit MMA input type), as the
-// reference does (AttentionKernel+Softmax.swift:304-324 sums P after the cast to its register type): rows of P / l then
-// sum to one exactly, whatever the rounding did.
-#ifndef MFA_SUM_ROUNDED_P
-#define MFA_SUM_ROUNDED_P 0
-#endif
-constexpr bool kSumRoundedP = MFA_SUM_ROUNDED_P != 0;
-// Pairs by which "sum and pack" trails "exp2" in softmax_exp_half.  A warp issues in order: with the consumer of an
-// ex2 right behind it (what a plain loop compiles to) every pair exposes the MUFU latency -- measured 26 cycles per
-// pair against the pipe's 16 (two ex2 at 4 lanes / clk / sub-partition).
-#ifndef MFA_EXP_SKEW
-#define MFA_EXP_SKEW 4
-#endif
 
 // One half-row (64 scores, FP32 bits in v) -> P = exp2(s * scale_log2 - m) rounded to 16 bits in `packed`; returns the
 // half-row sum.  v is consumed in place.  kPolyPairs of every 4 element pairs take exp2 on the FMA pipe (exp2_poly2)
 // instead of the MUFU pipe.
 template <bool kBF16, uint32_t kPolyPairs>
 __device__ __forceinline__ float softmax_exp_half(uint32_t (&v)[64], uint32_t (&packed)[32], float scale_log2, float m) {
-  constexpr uint32_t kSkew = MFA_EXP_SKEW;
+  // Pairs by which "sum and pack" trails "exp2".  A warp issues in order: with the consumer of an ex2 right behind it
+  // (what a plain loop compiles to) every pair exposes the MUFU latency -- measured 26 cycles per pair against the
+  // pipe's 16 (two ex2 at 4 lanes / clk / sub-partition).
+  constexpr uint32_t kSkew = 4;
   const float2 scale2 = make_float2(scale_log2, scale_log2), negm2 = make_float2(-m, -m);
   float2 acc0 = make_float2(0.f, 0.f), acc1 = make_float2(0.f, 0.f);
 #pragma unroll
@@ -403,7 +393,6 @@ __device__ __forceinline__ float softmax_exp_half(uint32_t (&v)[64], uint32_t (&
       const uint32_t k = i - kSkew;
       float2 e = make_float2(__uint_as_float(v[2 * k]), __uint_as_float(v[2 * k + 1]));
       packed[k] = kBF16 ? pack_bf16x2(e.x, e.y) : pack_f16x2(e.x, e.y);
-      if (kSumRoundedP) e = kBF16 ? unpack_bf16x2(packed[k]) : unpack_f16x2(packed[k]);
       if (k & 1)
         acc1 = fadd2(acc1, e);
       else

@@ -30,12 +30,6 @@
 #include "sm100_ptx.cuh"
 #include "tma_host.h"
 
-// 1: the persistent dQ kernel's D = rowsum(dO * O) is computed one item ahead by warp 11 (0: by the elementwise warps at
-// the head of every item, as in the one-item-per-CTA form); A/B builds: make VARIANT=inlineD EXTRA=-DMFA_DQ_DTERM_OFFLOAD=0
-#ifndef MFA_DQ_DTERM_OFFLOAD
-#define MFA_DQ_DTERM_OFFLOAD 1
-#endif
-
 namespace mfa {
 namespace bwd {
 
@@ -1097,7 +1091,7 @@ cudaError_t launch(const AttentionParams &p, cudaStream_t stream, bool key_value
   // head of an item that the offload removes matters for short items; the 48 KB staging area it needs costs long items ~4 %
   // (also with the offload switched off at run time, and with no-allocate loads: it is the shared-memory footprint, 225
   // instead of 177 KB), so the two forms are separate instantiations and long items take the inline one.
-  if constexpr (QueryConfig<DPAD>::kPersistent && MFA_DQ_DTERM_OFFLOAD != 0) {
+  if constexpr (QueryConfig<DPAD>::kPersistent) {
     if (!key_value && per <= 24) {
       kernel_q = attention_backward_query_tcgen05<DPAD, kBF16, kConvertDO, kPoly, true>;
       smem_q = QueryConfig<DPAD, true>::kSmemBytes;
@@ -1158,7 +1152,7 @@ cudaError_t launch(const AttentionParams &p, cudaStream_t stream, bool key_value
   const uint32_t tensors = key_value ? 2 : 1;
   void *ws = nullptr;
   if ((e = workspace_for(device, stream, splits * tensors * tensor_elems * sizeof(float), &ws)) != cudaSuccess) return e;
-  float *scratch = reinterpret_cast<float *>(static_cast<char *>(ws) + kWorkspaceCounterBytes);
+  float *scratch = static_cast<float *>(ws);
   a.split_stride = tensors * tensor_elems;
   a.dQ = scratch;
   a.dV = scratch;
@@ -1191,24 +1185,13 @@ bool tcgen05_backward_supported(const AttentionParams &p) {
   return types && layout && p.D % 8 == 0 && p.D <= tcgen05_backward_max_head();
 }
 
-// D > 128 or any transposed operand: the layout-generic kernels
-static bool needs_generic(const AttentionParams &p) {
-  return p.D > 128 || p.transposed[sQ] || p.transposed[sK] || p.transposed[sV] || p.transposed[sO] || p.transposed[sdO] ||
-         p.transposed[sdQ] || p.transposed[sdK] || p.transposed[sdV];
-}
-
 // dK/dV, FP16 Q/K/V beside BF16 dO: convert dO in a pass of its own when the key tiles fill more than one wave of SMs
 bool tcgen05_backward_converts_dO_first(uint32_t C, uint32_t batch) {
   const uint64_t tiles = static_cast<uint64_t>((C + bwd::kTile - 1) / bwd::kTile) * batch;
   return tiles > static_cast<uint64_t>(device_sm_count(current_device()));
 }
 
-static cudaError_t launch_backward(const AttentionParams &p, cudaStream_t stream, bool key_value) {
-  if (!tcgen05_backward_supported(p)) {
-    set_launch_detail("descriptor is outside the tcgen05 backward kernels' domain");
-    return cudaErrorInvalidValue;
-  }
-  if (needs_generic(p)) return launch_tcgen05_backward_generic(p, stream, key_value);
+cudaError_t launch_tcgen05_backward(const AttentionParams &p, cudaStream_t stream, bool key_value) {
   const bool bf16 = p.prec[sQ] == BF16;
   const bool convert = p.prec[sdO] != p.prec[sQ];  // FP16 Q/K/V with BF16 dO
   // dK/dV with the reference's policy: every streamed dO block has to be rewritten as FP16 by two helper warps before
@@ -1222,11 +1205,10 @@ static cudaError_t launch_backward(const AttentionParams &p, cudaStream_t stream
     void *ws = nullptr;
     cudaError_t e = workspace_for(current_device(), stream, elements * 2, &ws, /*slot=*/2);
     if (e != cudaSuccess) return e;
-    void *converted = static_cast<char *>(ws) + kWorkspaceCounterBytes;
-    if ((e = launch_bf16_to_f16(p.buf[sdO], converted, elements, stream)) != cudaSuccess) return e;
-    q.buf[sdO] = converted;
+    if ((e = launch_bf16_to_f16(p.buf[sdO], ws, elements, stream)) != cudaSuccess) return e;
+    q.buf[sdO] = ws;
     q.prec[sdO] = q.prec[sQ];
-    return launch_backward(q, stream, key_value);
+    return launch_tcgen05_backward(q, stream, key_value);
   }
   // the row's exp2 column selects the instantiation (kernel creation has checked the range)
 #define MFA_BWD_MODES(DPAD_, POLY_)                                                          \
@@ -1248,13 +1230,6 @@ static cudaError_t launch_backward(const AttentionParams &p, cudaStream_t stream
 #undef MFA_BWD_MODES
 }
 
-cudaError_t launch_tcgen05_backward_query(const AttentionParams &p, cudaStream_t stream) {
-  return launch_backward(p, stream, false);
-}
-cudaError_t launch_tcgen05_backward_key_value(const AttentionParams &p, cudaStream_t stream) {
-  return launch_backward(p, stream, true);
-}
-
 // 1 launch, or 2 (kernel + sum_splits) when the traversal split engages for this problem size
 uint32_t tcgen05_backward_launch_count(int type, uint32_t R, uint32_t C, uint32_t batch, uint32_t min_blocks,
                                        uint32_t max_splits, bool convert_dO) {
@@ -1269,7 +1244,7 @@ void tcgen05_backward_geometry(int type, uint32_t D, uint32_t *threads, uint32_t
                                uint32_t *trav, uint32_t *head) {
   *threads = bwd::kThreads;
   if (type == 1)  // MFA_BACKWARD_QUERY
-    *smem_bytes = D <= 64 ? bwd::QueryConfig<64, MFA_DQ_DTERM_OFFLOAD != 0>::kSmemBytes  // (the larger of its two forms)
+    *smem_bytes = D <= 64 ? bwd::QueryConfig<64, true>::kSmemBytes  // (the larger of its two forms)
                           : bwd::QueryConfig<128>::kSmemBytes;
   else
     *smem_bytes = D <= 64 ? bwd::KeyValueConfig<64>::kSmemBytes : bwd::KeyValueConfig<128>::kSmemBytes;

@@ -614,7 +614,7 @@ cudaError_t launch_pass(const AttentionParams &p, cudaStream_t stream) {
   constexpr uint32_t tensors = kMode == kKeyValue ? 2 : 1;  // partial accumulators: [split][tensor][batch][rows][D]
   void *ws = nullptr;
   if ((e = workspace_for(device, stream, splits * tensors * tensor_elems * sizeof(float), &ws)) != cudaSuccess) return e;
-  float *scratch = reinterpret_cast<float *>(static_cast<char *>(ws) + kWorkspaceCounterBytes);
+  float *scratch = static_cast<float *>(ws);
   a.split_stride = tensors * tensor_elems;
   a.out = scratch;
   a.out2 = scratch + tensor_elems;
@@ -662,9 +662,8 @@ cudaError_t launch_tcgen05_backward_generic(const AttentionParams &p_in, cudaStr
     void *ws = nullptr;
     cudaError_t e = workspace_for(current_device(), stream, elements * 2, &ws, /*slot=*/2);
     if (e != cudaSuccess) return e;
-    void *converted = static_cast<char *>(ws) + kWorkspaceCounterBytes;
-    if ((e = launch_bf16_to_f16(p.buf[sdO], converted, elements, stream)) != cudaSuccess) return e;
-    p.buf[sdO] = converted;
+    if ((e = launch_bf16_to_f16(p.buf[sdO], ws, elements, stream)) != cudaSuccess) return e;
+    p.buf[sdO] = ws;
     p.prec[sdO] = p.prec[sQ];
   }
   const bool bf16 = p.prec[sQ] == BF16;

@@ -29,32 +29,16 @@
 #include "sm100_ptx.cuh"
 #include "tma_host.h"
 
-// 1: O leaves the kernel through TMA stores (0: generic-proxy stores from registers; A/B: make VARIANT=stg EXTRA=-DMFA_FWD_TMA_STORE=0)
-// K / V ring depth at D <= 64.  A/B on one box (profiles/r2_sweep_fwd_stages_d64.jsonl, TFLOP/s, 4 | 3 | 2 stages): N=4096
-// 757 | 767 | 757, N=2048 714 | 716 | 713, N=512 532 | 541 | 530: depth barely matters (the softmax warps set the pace), three
-// stages are never worse and free 32 KB of shared memory.
-#ifndef MFA_FWD_STAGES_D64
-#define MFA_FWD_STAGES_D64 3
-#endif
-#ifndef MFA_FWD_TMA_STORE
-#define MFA_FWD_TMA_STORE 1
-#endif
-
 namespace mfa {
-// Split-KV has two forms (tests cover both; mfa_debug_set_forward_fused() selects):
-//   scratch -- TWO launches (default): normalised partials in the library's workspace + the combine_splits kernel,
-//              launched with programmatic stream serialisation so that it is resident when the attention kernel drains;
-//   fused   -- ONE launch: every split CTA leaves its raw partial (unnormalised O, m, l) in the workspace, announces it
-//              on a per-tile-pair arrival counter, waits for its siblings and then merges and stores a 1 / num_splits
-//              slice of the pair's rows (all CTAs are co-resident: cooperative launch, one item each).
-// Measured on B200, one N = 4096, D = 128 bf16 head (profiles/r2_single_head_latency.jsonl), eager / CUDA graph:
-// scratch 20.5 / 18.3 us, fused 22.6 / 20.5 us -- the merge is the same L2 traffic either way, and the second launch
-// (hidden behind the first by programmatic stream serialisation) costs less than the cooperative launch plus the
-// arrive-and-spin round trip, so the one-launch form is not the default.  A third form that reduced through
-// distributed shared memory inside a thread-block cluster was measured at 37 us in round 1 (only 15 clusters of 8 CTAs
-// are co-resident, DSMEM pulls at ~6 B/clk/SM) and removed.
-static int g_forward_fused_enabled = 0;
-void tcgen05_forward_set_fused(int enabled) { g_forward_fused_enabled = enabled; }
+// Split-KV takes two launches: normalised partials in the library's workspace, then the combine_splits kernel, launched
+// with programmatic stream serialisation so that it is resident when the attention kernel drains.  A one-launch form
+// (every split CTA left its raw partial in the workspace, waited on a per-tile-pair arrival counter for its siblings
+// and merged a slice of the rows; cooperative launch) measured slower on B200, one N = 4096, D = 128 bf16 head
+// (profiles/r2_single_head_latency.jsonl), eager / CUDA graph: two launches 20.5 / 18.3 us, one launch 22.6 / 20.5 us --
+// the merge is the same L2 traffic either way, and the second launch (hidden behind the first by programmatic stream
+// serialisation) costs less than the cooperative launch plus the arrive-and-spin round trip.  It was removed, as was a
+// form that reduced through distributed shared memory inside a thread-block cluster (37 us in round 1: only 15
+// clusters of 8 CTAs are co-resident, DSMEM pulls at ~6 B/clk/SM).
 
 namespace fwd {
 
@@ -75,17 +59,16 @@ static_assert(kSoftmaxRegs * 256 + kOtherRegs * 128 <= kLaunchRegs * kThreads, "
 // scripts/sweep.py repeats it):  D=128: 0 -> 1258, 1 -> 1241, 2 -> 1183;  D=64: 0 -> 729, 1 -> 765, 2 -> 737.  At D = 64
 // the tensor pipe needs half as long per block, the MUFU pipe (16 ex2 / clk / SM) just as long, so taking a quarter of the
 // exponentials off it pays; at D = 128 it only costs issue slots.
-constexpr float kLazySumLimit = 256.0f;
-#ifndef MFA_FWD_WARP_ARRIVE
-#define MFA_FWD_WARP_ARRIVE 0
-#endif
-constexpr bool kWarpArrive = MFA_FWD_WARP_ARRIVE != 0;  // P hand-off: one mbarrier arrival per softmax warp, not per thread  // a half-row of P summing to <= 2^8 proves every element is <= 2^8
+constexpr float kLazySumLimit = 256.0f;  // a half-row of P summing to <= 2^8 proves every element is <= 2^8
 
 template <uint32_t DPAD>
 struct Config {
   static constexpr uint32_t kSubTiles = DPAD / 64;                 // 64-element sub-tiles along D
   static constexpr uint32_t kTileBytes = kSubTiles * kSubTileBytes;  // one 128 x DPAD operand tile
-  static constexpr uint32_t kStages = DPAD <= 64 ? MFA_FWD_STAGES_D64 : 2;
+  // K / V ring depth.  At D <= 64, A/B on one box (profiles/r2_sweep_fwd_stages_d64.jsonl, TFLOP/s, 4 | 3 | 2 stages):
+  // N=4096 757 | 767 | 757, N=2048 714 | 716 | 713, N=512 532 | 541 | 530: depth barely matters (the softmax warps set the
+  // pace), three stages are never worse and free 32 KB of shared memory.
+  static constexpr uint32_t kStages = DPAD <= 64 ? 3 : 2;
   static constexpr uint32_t kSmemQ = 0;
   static constexpr uint32_t kSmemK = kSmemQ + kTilesPerCta * kTileBytes;
   static constexpr uint32_t kSmemV = kSmemK + kStages * kTileBytes;
@@ -116,15 +99,14 @@ constexpr uint32_t kTraceSlots = 8;  // per (role, iteration)
 // item-level probes: roles 4 (tile 0 softmax), 5 (tile 1 softmax), 6 (MMA), indexed by the CTA's item counter
 #define MFA_TRACE_ITEM(role, it, slot) MFA_TRACE(role, it, slot)
 
-template <uint32_t DPAD, bool kBF16, uint32_t kPolyPairs, bool kTrace = false, bool kFused = false, bool kTmaStoreO = false>
+template <uint32_t DPAD, bool kBF16, uint32_t kPolyPairs, bool kTrace = false, bool kTmaStoreO = false>
 __global__ void __launch_bounds__(kThreads, 1)
     attention_forward_tcgen05(const __grid_constant__ CUtensorMap mapQ, const __grid_constant__ CUtensorMap mapK,
                               const __grid_constant__ CUtensorMap mapV, const __grid_constant__ CUtensorMap mapO,
                               float *__restrict__ O, void *__restrict__ L,
                               uint32_t R, uint32_t C, uint32_t D, float scale_log2, int l_is_fp16,
                               uint32_t num_items, uint32_t pairs_per_head, uint32_t num_splits, uint32_t batch,
-                              float *__restrict__ part_O, float2 *__restrict__ part_ml,
-                              uint32_t *__restrict__ counters, long long *__restrict__ trace) {
+                              long long *__restrict__ trace) {
   // Persistent CTAs: one per SM, each walking the work items (head, 256-row tile pair) blockIdx.x,
   // blockIdx.x + gridDim.x, ...  Barrier phases are carried across items, so the producers (TMA, MMA) run ahead
   // into the next item while the softmax warps drain the current one; TMEM alloc, barrier init and descriptor
@@ -135,13 +117,9 @@ __global__ void __launch_bounds__(kThreads, 1)
 
   const uint32_t warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
   // Split-KV: when there are fewer (head, tile pair) items than SMs, the key axis of every item is cut into
-  // num_splits equal ranges that become separate work items.
-  //  kFused: every CTA has exactly one item (cooperative launch: all are co-resident).  It leaves its raw partial --
-  //    unnormalised O, running max m and sum l -- in the workspace ([pair][split][256 rows]), bumps the pair's
-  //    arrival counter, waits until all num_splits siblings have arrived and then merges and stores the rows
-  //    [split * 256 / num_splits, ...) of the pair: one launch, and the merge is spread over all split CTAs.
-  //  otherwise (fallback): each item writes a normalised partial O and its L as if it were a whole problem (O and L
-  //    then point at scratch laid out [split][head][row]) and the combine_splits kernel merges them.
+  // num_splits equal ranges that become separate work items.  Each writes a normalised partial O and its L as if it
+  // were a whole problem (O and L then point at scratch laid out [split][head][row]) and the combine_splits kernel
+  // merges them.
   const uint32_t total_blocks = (C + kBlockN - 1) / kBlockN;
   const uint32_t num_blocks = total_blocks / num_splits;  // key blocks per work item (host guarantees divisibility)
 
@@ -172,8 +150,8 @@ __global__ void __launch_bounds__(kThreads, 1)
     }
     for (uint32_t t = 0; t < kTilesPerCta; ++t) {
       mbar_init(&b.s_full[t], 1);
-      mbar_init(&b.p_full[2 * t], kWarpArrive ? kTileM / 32 : kTileM);
-      mbar_init(&b.p_full[2 * t + 1], kWarpArrive ? kTileM / 32 : kTileM);
+      mbar_init(&b.p_full[2 * t], kTileM);
+      mbar_init(&b.p_full[2 * t + 1], kTileM);
       mbar_init(&b.o_full[t], 1);
       mbar_init(&b.o_free[t], kTileM);
       mbar_init(&b.pv_half[t], 1);
@@ -193,9 +171,9 @@ __global__ void __launch_bounds__(kThreads, 1)
   __syncthreads();
   tc_fence_after();
   const uint32_t tmem_base = *tmem_ptr_smem;
-  // scratch split-KV: let the combine kernel (launched with programmatic stream serialisation) be set up now; its
+  // split-KV: let the combine kernel (launched with programmatic stream serialisation) be set up now; its
   // griddepcontrol.wait still holds it until this grid has completed and flushed
-  if (!kFused && num_splits > 1) asm volatile("griddepcontrol.launch_dependents;" ::: "memory");
+  if (num_splits > 1) asm volatile("griddepcontrol.launch_dependents;" ::: "memory");
 
   if (warp < 8) {
     // =====================================================================================
@@ -212,8 +190,8 @@ __global__ void __launch_bounds__(kThreads, 1)
 
     for (uint32_t item = blockIdx.x, it = 0; item < num_items; item += gridDim.x, ++it) {
     const uint32_t split = item % num_splits;
-    // output slot; the scratch fallback lays partials out as [split][head]
-    const uint32_t head = (item / num_splits) / pairs_per_head + (kFused ? 0u : split * batch);
+    // output slot; split-KV lays partials out as [split][head]
+    const uint32_t head = (item / num_splits) / pairs_per_head + split * batch;
     const uint32_t q_row0 = ((item / num_splits) % pairs_per_head) * (kTileM * kTilesPerCta);
     const uint32_t key_block0 = split * num_blocks;
     const uint32_t g0 = it * num_blocks;  // key blocks this CTA has processed before this item (barrier phases)
@@ -269,7 +247,6 @@ __global__ void __launch_bounds__(kThreads, 1)
               pr.y = ex2_approx(x.y);
             }
             packed[i] = kBF16 ? pack_bf16x2(pr.x, pr.y) : pack_f16x2(pr.x, pr.y);
-            if (kSumRoundedP) pr = kBF16 ? unpack_bf16x2(packed[i]) : unpack_f16x2(packed[i]);
             sum2 = fadd2(sum2, pr);
           }
           half_sum = sum2.x + sum2.y;
@@ -312,14 +289,8 @@ __global__ void __launch_bounds__(kThreads, 1)
             const float p0 = ex2_approx(fmaf(s[c0 + 2 * i], scale_log2, -m));
             const float p1 = ex2_approx(fmaf(s[c0 + 2 * i + 1], scale_log2, -m));
             packed[i] = kBF16 ? pack_bf16x2(p0, p1) : pack_f16x2(p0, p1);
-            if (kSumRoundedP) {
-              const float2 q = kBF16 ? unpack_bf16x2(packed[i]) : unpack_f16x2(packed[i]);
-              sum0 += q.x;
-              sum1 += q.y;
-            } else {
-              sum0 += p0;
-              sum1 += p1;
-            }
+            sum0 += p0;
+            sum1 += p1;
           }
           half_sum = sum0 + sum1;
         }
@@ -330,14 +301,7 @@ __global__ void __launch_bounds__(kThreads, 1)
         tc_fence_before();
         // the first 64 columns of P are released on their own so that the MMA warp starts O += P V on them while
         // the MUFU pipe works through the other half
-        if (kWarpArrive) {
-          // one arrival per warp: tcgen05.wait::st is warp-collective, so once the warp has passed it (and
-          // synchronised) every lane's stores are complete; 4 arrivals instead of 128 reach the MMA warp sooner
-          __syncwarp();
-          if (lane == 0) mbar_arrive(&b.p_full[2 * t + half]);
-        } else {
-          mbar_arrive(&b.p_full[2 * t + half]);
-        }
+        mbar_arrive(&b.p_full[2 * t + half]);
         MFA_TRACE(warp == 0 ? 0 : (warp == 4 ? 1 : 5), j, 2 + half);
       }
       MFA_TRACE(warp == 0 ? 0 : (warp == 4 ? 1 : 5), j, 4);
@@ -345,37 +309,30 @@ __global__ void __launch_bounds__(kThreads, 1)
 
     {
       // ---------------- epilogue: O / l -> global (FP32), L = m + log2(l) ----------------
-      // (fused split-KV: the RAW accumulator -> this split's slot of the workspace instead, then the merge below)
       MFA_TRACE_ITEM(warp == 0 ? 4 : (warp == 4 ? 5 : 7), it, 1);
       mbar_wait(&b.o_full[t], (g0 + num_blocks - 1) & 1);
       tc_fence_after();
       MFA_TRACE_ITEM(warp == 0 ? 4 : (warp == 4 ? 5 : 7), it, 2);
       const uint32_t row = q_row0 + t * kTileM + row_in_tile;
-      const uint32_t pair_item = item / num_splits;  // (head, tile pair)
-      const float out_scale = kFused ? 1.0f : 1.0f / l;
+      const float out_scale = 1.0f / l;
       // TMEM hands every thread one row; storing rows straight from registers would touch 32 different cache
       // lines per warp store.  Each warp therefore transposes 32 x 32 chunks through a private XOR-swizzled scratch
       // tile in shared memory (128-bit accesses, conflict-free both ways) and writes four full 128 B lines per store.
       const uint32_t scratch = smem_u32(smem + Cfg::kSmemScratch) + warp * (32 * 8 * 16);  // this warp's 4 KB tile
       const uint32_t warp_row0 = q_row0 + t * kTileM + (warp & 3) * 32;
-      // rows the stores may touch: the problem's R rows, or all 256 slots of the pair in the workspace
-      const uint32_t row_limit = kFused ? q_row0 + kTileM * kTilesPerCta : R;
-      float *o_base = kFused ? part_O + ((static_cast<size_t>(pair_item) * num_splits + split) * (kTileM * kTilesPerCta) +
-                                         (t * kTileM + (warp & 3) * 32)) * D
-                             : O + (static_cast<size_t>(head) * R + warp_row0) * D;
+      float *o_base = O + (static_cast<size_t>(head) * R + warp_row0) * D;
       const uint32_t sub_row = lane >> 3, quad = lane & 7;  // transposed view: 4 rows x 8 float4 per warp access
-      // Non-fused form: the transposed chunk leaves through the TMA (cp.async.bulk.tensor store from the scratch tile,
+      // Short items: the transposed chunk leaves through the TMA (cp.async.bulk.tensor store from the scratch tile,
       // whose XOR pattern IS the 128-byte swizzle of a [32 rows][32 floats] box): the warp does not wait for the global
       // writes -- it only waits, before rewriting the scratch tile, until the previous chunk's store has READ it.  Rows past
-      // R and columns past D are clipped by the tensor map.  (Generic-proxy stores from registers, the fused form below,
-      // held the warp until every line had left the SM.)  With one scratch tile per warp the wait for the previous chunk's
+      // R and columns past D are clipped by the tensor map.  (Generic-proxy stores from registers, the other instantiation,
+      // hold the warp until every line has left the SM.)  With one scratch tile per warp the wait for the previous chunk's
       // read is partly exposed, and at 32 blocks per item the epilogue is too small a share to matter, so the launcher picks
       // this instantiation for short items only (A/B on one box, TFLOP/s, this build | register stores: N=512 D=64 525 | 501,
       // N=1024 D=128 833 | 780, N=2048 D=64 FP16 712 | 702; N=4096 D=128 equal: profiles/r2_sweep_fwd_tma_store.jsonl).
       // (A second scratch tile per warp at D <= 64, so that the two chunks never wait for each other, measured the same
       // within 0.5 %: profiles/r2_sweep_fwd_two_tiles.jsonl -- not kept.)
       constexpr bool kTmaStore = kTmaStoreO;  // (its own instantiation: as a run-time branch it cost the long-item case 1.8 %)
-      static_assert(!(kFused && kTmaStoreO), "the fused form keeps the register stores");
   #pragma unroll
       for (uint32_t c = 0; c < DPAD; c += 32) {
         uint32_t o[32];
@@ -412,101 +369,19 @@ __global__ void __launch_bounds__(kThreads, 1)
   #pragma unroll
             for (uint32_t i = 0; i < 8; ++i) {
               const uint32_t r = 4 * i + sub_row;
-              if (warp_row0 + r < row_limit) *reinterpret_cast<float4 *>(o_base + static_cast<size_t>(r) * D + c + 4 * quad) = v[i];
+              if (warp_row0 + r < R) *reinterpret_cast<float4 *>(o_base + static_cast<size_t>(r) * D + c + 4 * quad) = v[i];
             }
           }
           __syncwarp();
         }
       }
-      if constexpr (!kFused) {
-        if (row < R && L != nullptr) {
-          const float lse2 = m + log2f(l);  // AttentionKernel+Caching.swift:373-377
-          const size_t idx = static_cast<size_t>(head) * R + row;
-          if (l_is_fp16)
-            reinterpret_cast<__half *>(L)[idx] = __float2half_rn(lse2);
-          else
-            reinterpret_cast<float *>(L)[idx] = lse2;
-        }
-      } else {
-        // ---------------- fused split-KV: publish the partial, wait for the siblings, merge a slice of the rows ------
-        constexpr uint32_t kPairRows = kTileM * kTilesPerCta;
-        const size_t slot0 = static_cast<size_t>(pair_item) * num_splits * kPairRows;  // first row slot of this pair
-        part_ml[slot0 + static_cast<size_t>(split) * kPairRows + t * kTileM + row_in_tile] = make_float2(m, l);
-        __threadfence();  // the partial is visible device-wide before the arrival is
-        asm volatile("bar.sync 1, 256;" ::: "memory");  // the eight softmax warps
-        uint32_t *arrived = counters + 2 * pair_item, *merged = arrived + 1;
-        if (threadIdx.x == 0) {
-          atomicAdd(arrived, 1u);
-          // bounded spin (a protocol bug must trap, not hang): the siblings are co-resident, so this is short
-          const long long start = clock64();
-          uint32_t seen;
-          do {
-            asm volatile("ld.acquire.gpu.global.u32 %0, [%1];" : "=r"(seen) : "l"(arrived) : "memory");
-            if (seen < num_splits && clock64() - start > MFA_MBAR_TIMEOUT_CYCLES) {
-              printf("mfa_b200: split-KV arrival timeout block %d (%u of %u)\n", blockIdx.x, seen, num_splits);
-              __trap();
-            }
-          } while (seen < num_splits);
-        }
-        asm volatile("bar.sync 1, 256;" ::: "memory");
-        MFA_TRACE_ITEM(warp == 0 ? 4 : (warp == 4 ? 5 : 7), it, 4);
-        // rows [split * rows_per_rank, ...) of the pair: thread <-> (row, 16 B column slot), DPAD / 4 consecutive threads
-        // per row, so the global stores are full lines; every load of a thread is issued before the first use
-        constexpr uint32_t kQuadsPerRow = DPAD / 4;
-        const uint32_t rows_per_rank = (kPairRows + num_splits - 1) / num_splits;
-        const uint32_t mq = threadIdx.x % kQuadsPerRow;
-        for (uint32_t r = threadIdx.x / kQuadsPerRow; r < rows_per_rank; r += 256 / kQuadsPerRow) {
-          const uint32_t rt = split * rows_per_rank + r;
-          if (rt >= kPairRows) break;
-          float2 mls[16];
-          float4 vs[16];
-#pragma unroll
-          for (uint32_t sp = 0; sp < 16; ++sp) {
-            mls[sp] = make_float2(-FLT_MAX, 0.f);
-            vs[sp] = make_float4(0.f, 0.f, 0.f, 0.f);
-            if (sp < num_splits) {
-              const size_t slot = slot0 + static_cast<size_t>(sp) * kPairRows + rt;
-              mls[sp] = __ldcg(part_ml + slot);
-              if (4 * mq < D) vs[sp] = __ldcg(reinterpret_cast<const float4 *>(part_O + slot * D) + mq);
-            }
-          }
-          float m_all = -FLT_MAX;
-#pragma unroll
-          for (uint32_t sp = 0; sp < 16; ++sp) m_all = fmaxf(m_all, mls[sp].x);
-          float denom = 0.f;
-          float4 acc = make_float4(0.f, 0.f, 0.f, 0.f);
-#pragma unroll
-          for (uint32_t sp = 0; sp < 16; ++sp) {
-            const float w = exp2f(mls[sp].x - m_all);  // unused slots: l = 0 and O = 0, so their weight is irrelevant
-            denom = fmaf(w, mls[sp].y, denom);
-            acc.x = fmaf(w, vs[sp].x, acc.x);
-            acc.y = fmaf(w, vs[sp].y, acc.y);
-            acc.z = fmaf(w, vs[sp].z, acc.z);
-            acc.w = fmaf(w, vs[sp].w, acc.w);
-          }
-          const float inv = 1.0f / denom;
-          const uint32_t out_row = q_row0 + rt;
-          if (out_row < R) {
-            if (4 * mq < D)
-              *reinterpret_cast<float4 *>(O + (static_cast<size_t>(head) * R + out_row) * D + 4 * mq) =
-                  make_float4(acc.x * inv, acc.y * inv, acc.z * inv, acc.w * inv);
-            if (mq == 0 && L != nullptr) {
-              const float lse2 = m_all + log2f(denom);  // AttentionKernel+Caching.swift:373-377
-              const size_t idx = static_cast<size_t>(head) * R + out_row;
-              if (l_is_fp16)
-                reinterpret_cast<__half *>(L)[idx] = __float2half_rn(lse2);
-              else
-                reinterpret_cast<float *>(L)[idx] = lse2;
-            }
-          }
-        }
-        // the last CTA to finish reading returns both counters to zero for the next launch on this stream
-        asm volatile("bar.sync 1, 256;" ::: "memory");
-        if (threadIdx.x == 0 && atomicAdd(merged, 1u) == num_splits - 1) {
-          *arrived = 0;
-          *merged = 0;
-        }
-        MFA_TRACE_ITEM(warp == 0 ? 4 : (warp == 4 ? 5 : 7), it, 5);
+      if (row < R && L != nullptr) {
+        const float lse2 = m + log2f(l);  // AttentionKernel+Caching.swift:373-377
+        const size_t idx = static_cast<size_t>(head) * R + row;
+        if (l_is_fp16)
+          reinterpret_cast<__half *>(L)[idx] = __float2half_rn(lse2);
+        else
+          reinterpret_cast<float *>(L)[idx] = lse2;
       }
     }
     // O of this tile is out of TMEM: the next item's first O = P V (accumulate off) may overwrite it
@@ -676,7 +551,7 @@ __global__ void __launch_bounds__(kThreads, 1)
   }
 }
 
-// Merges the num_splits partial results of split-KV (scratch form): L = log2 sum_s 2^L_s,  O = sum_s 2^(L_s - L) O_s.
+// Merges the num_splits partial results of split-KV: L = log2 sum_s 2^L_s,  O = sum_s 2^(L_s - L) O_s.
 // One thread per (row, 4 columns); partials are [split][head][row][D] FP32 and [split][head][row] FP32.  Every load of
 // a thread is issued before the first use (the partials sit in L2; a dependent chain of num_splits round trips was
 // 3x slower).  Launched with programmatic stream serialisation: the grid is set up while the attention kernel drains
@@ -744,7 +619,7 @@ static uint32_t choose_splits(uint32_t items, uint32_t total_blocks, uint32_t sm
 template <uint32_t DPAD, bool kBF16, uint32_t kPoly, bool kTrace = false>
 cudaError_t launch(const AttentionParams &p, cudaStream_t stream, long long *trace = nullptr) {
   using Cfg = Config<DPAD>;
-  auto kernel = attention_forward_tcgen05<DPAD, kBF16, kPoly, kTrace, false, false>;
+  auto kernel = attention_forward_tcgen05<DPAD, kBF16, kPoly, kTrace, false>;
   const int device = current_device();
   cudaError_t e;
   if ((e = ensure_max_dynamic_smem(reinterpret_cast<const void *>(kernel), Cfg::kSmemBytes, device)) != cudaSuccess) return e;
@@ -763,9 +638,9 @@ cudaError_t launch(const AttentionParams &p, cudaStream_t stream, long long *tra
   const uint32_t splits = choose_splits(num_items, total_blocks, sm_count, p.split_min_blocks, p.split_max);
   // short items (many epilogues per unit of work): O leaves through TMA stores; long items keep the register stores
   // (split single heads measured 1-2 % slower with it: one item per CTA, nothing to overlap the store with)
-  if constexpr (MFA_FWD_TMA_STORE != 0 && !kTrace) {
+  if constexpr (!kTrace) {
     if (splits == 1 && total_blocks <= 16) {
-    kernel = attention_forward_tcgen05<DPAD, kBF16, kPoly, kTrace, false, true>;
+    kernel = attention_forward_tcgen05<DPAD, kBF16, kPoly, kTrace, true>;
     if ((e = ensure_max_dynamic_smem(reinterpret_cast<const void *>(kernel), Cfg::kSmemBytes, device)) != cudaSuccess) return e;
     }
   }
@@ -774,56 +649,25 @@ cudaError_t launch(const AttentionParams &p, cudaStream_t stream, long long *tra
     const uint32_t grid = num_items < sm_count ? num_items : sm_count;
     kernel<<<grid, kThreads, Cfg::kSmemBytes, stream>>>(mapQ, mapK, mapV, mapO, static_cast<float *>(p.buf[sO]), p.buf[sL],
                                                         p.R, p.C, p.D, p.scale_log2, l_is_fp16, num_items,
-                                                        pairs_per_head, 1u, p.batch, nullptr, nullptr, nullptr, trace);
+                                                        pairs_per_head, 1u, p.batch, trace);
     return cudaGetLastError();
   }
 
-  // ---- split-KV: partials live in the library's per-(device, stream) workspace -----------------------------------
+  // ---- split-KV: normalised partial O / L per split ([split][head][row]) in the library's per-(device, stream)
+  // workspace, then the combine kernel
   const uint32_t split_items = num_items * splits;  // <= sm_count by construction of choose_splits
-  constexpr uint32_t kPairRows = kTileM * kTilesPerCta;
-  if (g_forward_fused_enabled && split_items <= sm_count && 2 * num_items * sizeof(uint32_t) <= kWorkspaceCounterBytes) {
-    // fused form: one cooperative launch (every CTA resident, one item each); [counters | O partials | (m, l)]
-    auto fused = attention_forward_tcgen05<DPAD, kBF16, kPoly, kTrace, true>;
-    if ((e = ensure_max_dynamic_smem(reinterpret_cast<const void *>(fused), Cfg::kSmemBytes, device)) != cudaSuccess) return e;
-    const size_t slots = static_cast<size_t>(split_items) * kPairRows;
-    const size_t o_bytes = slots * p.D * sizeof(float), ml_bytes = slots * sizeof(float2);
-    void *ws = nullptr;
-    if ((e = workspace_for(device, stream, o_bytes + ml_bytes, &ws)) != cudaSuccess) return e;
-    uint32_t *counters = static_cast<uint32_t *>(ws);
-    float *part_O = reinterpret_cast<float *>(static_cast<char *>(ws) + kWorkspaceCounterBytes);
-    float2 *part_ml = reinterpret_cast<float2 *>(reinterpret_cast<char *>(part_O) + o_bytes);
-    cudaLaunchAttribute attr;
-    attr.id = cudaLaunchAttributeCooperative;
-    attr.val.cooperative = 1;
-    cudaLaunchConfig_t config = {};
-    config.gridDim = dim3(split_items, 1, 1);
-    config.blockDim = dim3(kThreads, 1, 1);
-    config.dynamicSmemBytes = Cfg::kSmemBytes;
-    config.stream = stream;
-    config.attrs = &attr;
-    config.numAttrs = 1;
-    mapO = mapQ;  // (unused by the fused form)
-    e = cudaLaunchKernelEx(&config, fused, mapQ, mapK, mapV, mapO, static_cast<float *>(p.buf[sO]), p.buf[sL], p.R, p.C, p.D,
-                           p.scale_log2, l_is_fp16, split_items, pairs_per_head, splits, p.batch, part_O, part_ml,
-                           counters, trace);
-    if (e == cudaSuccess) return cudaGetLastError();
-    cudaGetLastError();  // cooperative launch refused (e.g. a partitioned GPU): fall through to the two-launch form
-  }
-
-  // scratch form: normalised partial O / L per split ([split][head][row]), then the combine kernel
   const uint64_t rows_total = static_cast<uint64_t>(p.batch) * p.R;
   const size_t o_bytes = static_cast<size_t>(splits) * rows_total * p.D * sizeof(float);
   const size_t l_bytes = static_cast<size_t>(splits) * rows_total * sizeof(float);
   void *ws = nullptr;
   if ((e = workspace_for(device, stream, o_bytes + l_bytes, &ws)) != cudaSuccess) return e;
-  float *scratch = reinterpret_cast<float *>(static_cast<char *>(ws) + kWorkspaceCounterBytes);
+  float *scratch = static_cast<float *>(ws);
   float *L_part = scratch + static_cast<size_t>(splits) * rows_total * p.D;
   // partials are laid out [split][head][row][D]: one tensor map over splits x batch "heads"
   if ((e = make_tensor_map_f32(&mapO, scratch, p.R, p.D, p.batch * splits, 32)) != cudaSuccess) return e;
   const uint32_t grid = split_items < sm_count ? split_items : sm_count;
   kernel<<<grid, kThreads, Cfg::kSmemBytes, stream>>>(mapQ, mapK, mapV, mapO, scratch, L_part, p.R, p.C, p.D, p.scale_log2,
-                                                      0, split_items, pairs_per_head, splits, p.batch, nullptr, nullptr,
-                                                      nullptr, trace);
+                                                      0, split_items, pairs_per_head, splits, p.batch, trace);
   if ((e = cudaGetLastError()) != cudaSuccess) return e;
   const uint64_t threads = rows_total * (p.D / 4);
   cudaLaunchAttribute attr;
@@ -859,14 +703,7 @@ bool tcgen05_forward_supported(const AttentionParams &p) {
 }
 
 cudaError_t launch_tcgen05_forward(const AttentionParams &p, cudaStream_t stream) {
-  if (!tcgen05_forward_supported(p)) {
-    set_launch_detail("descriptor is outside the tcgen05 forward kernel's domain");
-    return cudaErrorInvalidValue;
-  }
-  if (p.transposed[sQ] || p.transposed[sK] || p.transposed[sV] || p.transposed[sO])
-    return launch_tcgen05_forward_generic(p, stream);  // tcgen05_forward_d256.cu
   const bool bf16 = p.prec[sQ] == BF16;
-  if (p.D > 128) return launch_tcgen05_forward_d256(p, stream);  // tcgen05_forward_d256.cu
   // the row's exp2 column selects the instantiation (kernel creation has checked the range)
 #define MFA_FWD_DISPATCH(DPAD_)                                                                              \
   switch (p.exp2_fma_quarters) {                                                                             \
@@ -887,24 +724,16 @@ cudaError_t launch_tcgen05_forward_trace(const AttentionParams &p, cudaStream_t 
   return fwd::launch<128, true, 0, true>(p, stream, trace);
 }
 
-// 1 launch, or 2 (attention + combine) when the scratch form of split-KV engages for this problem size
-uint32_t tcgen05_forward_launch_count(uint32_t R, uint32_t C, uint32_t D, uint32_t batch, uint32_t min_blocks,
-                                      uint32_t max_splits) {
-  if (D > 128) return 1;
+// 1 launch, or 2 (attention + combine) when split-KV engages for this problem size
+uint32_t tcgen05_forward_launch_count(uint32_t R, uint32_t C, uint32_t batch, uint32_t min_blocks, uint32_t max_splits) {
   const uint32_t sm_count = device_sm_count(current_device());
   const uint32_t pairs = (R + fwd::kTileM * fwd::kTilesPerCta - 1) / (fwd::kTileM * fwd::kTilesPerCta);
   const uint32_t blocks = (C + fwd::kBlockN - 1) / fwd::kBlockN;
-  if (fwd::choose_splits(pairs * batch, blocks, sm_count, min_blocks, max_splits) == 1) return 1;
-  return g_forward_fused_enabled ? 1 : 2;  // fused split-KV merges inside the attention kernel
+  return fwd::choose_splits(pairs * batch, blocks, sm_count, min_blocks, max_splits) == 1 ? 1 : 2;
 }
 
 void tcgen05_forward_geometry(uint32_t D, uint32_t *threads, uint32_t *smem_bytes, uint32_t *par, uint32_t *trav,
                               uint32_t *head) {
-  if (D > 128) {
-    tcgen05_forward_d256_geometry(threads, smem_bytes, par, trav);
-    *head = 256 < (D + 7) / 8 * 8 ? 256 : (D + 7) / 8 * 8;
-    return;
-  }
   *threads = fwd::kThreads;
   *smem_bytes = D <= 64 ? fwd::Config<64>::kSmemBytes : fwd::Config<128>::kSmemBytes;
   *par = fwd::kTileM * fwd::kTilesPerCta;

@@ -562,11 +562,4 @@ cudaError_t launch_tcgen05_forward_d256(const AttentionParams &p, cudaStream_t s
   return p.prec[sQ] == BF16 ? fwd256::launch<256, true>(p, stream) : fwd256::launch<256, false>(p, stream);
 }
 
-void tcgen05_forward_d256_geometry(uint32_t *threads, uint32_t *smem_bytes, uint32_t *par, uint32_t *trav) {
-  *threads = fwd256::kThreads;
-  *smem_bytes = fwd256::Config<256>::kSmemBytes;
-  *par = fwd256::kTileM;
-  *trav = fwd256::kBlockN;
-}
-
 }  // namespace mfa

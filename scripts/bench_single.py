@@ -1,6 +1,6 @@
 """Single-head latency of the three kernels, device-timed two ways: an eager launch loop (includes whatever the host
 cannot hide) and a CUDA graph of the same launches (the launch-bound inner loop captured, as a serving stack would run
-it).  Forward is shown with split-KV in both forms (fused: one launch, merge inside the kernel; scratch + combine kernel).
+it).  Where split-KV engages, the forward is two launches (attention + combine kernel).
 Usage (GPU box):  python scripts/bench_single.py"""
 import json
 import os
@@ -65,19 +65,12 @@ def run(N, D, precision, H=1):
         if D > 128 and t != KT.forward:
             continue
         k = mfa.AttentionKernel(desc.kernelDescriptor(t))
-        forms = [("", 1)]
-        if t == KT.forward and D <= 128:
-            forms = [("fused", 1), ("scratch", 0)]
-        for name, flag in forms:
-            mfa._lib.mfa_debug_set_forward_fused(flag)
-            launches = k.launchCount(c)
-            eager_us, graph_us = time_kernel(k, c, ptrs)
-            fma, gemm = WORK[t]
-            key = t.name + ("/" + name if name else "")
-            out[key] = {"launches": launches, "eager_us": round(eager_us, 2), "graph_us": round(graph_us, 2),
-                        "tflops_graph": round(gemm * N * N * D * H / graph_us / 1e6, 1),
-                        "ginstrs_graph": round((fma * D + 5) * N * N * H / graph_us / 1e3, 1)}
-        mfa._lib.mfa_debug_set_forward_fused(0)
+        launches = k.launchCount(c)
+        eager_us, graph_us = time_kernel(k, c, ptrs)
+        fma, gemm = WORK[t]
+        out[t.name] = {"launches": launches, "eager_us": round(eager_us, 2), "graph_us": round(graph_us, 2),
+                       "tflops_graph": round(gemm * N * N * D * H / graph_us / 1e6, 1),
+                       "ginstrs_graph": round((fma * D + 5) * N * N * H / graph_us / 1e3, 1)}
     return out
 
 

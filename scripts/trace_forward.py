@@ -20,8 +20,6 @@ desc.inputPrecisionOverride = mfa.GEMMOperandPrecision.BF16
 desc.matrixDimensions = (R, C, D)
 desc.transposeState = (False,) * 4
 desc.batchCount = H
-if os.environ.get('MFA_NO_FUSED'):
-    mfa._lib.mfa_debug_set_forward_fused(0)
 kernel = mfa.AttentionKernel(desc.kernelDescriptor(mfa.AttentionKernelType.forward))
 constants = mfa.FunctionConstantValues()
 desc.setFunctionConstants(constants)
@@ -73,8 +71,8 @@ items = int((t[4, :, 0] != 0).sum())
 base = t[6, 0, 0]
 print(f"items processed by CTA 0: {items}; per item (cycles from the MMA warp's first prologue):")
 for it in range(min(items, 8)):
-    a = (t[4, it, :6] - base).tolist(); b2 = (t[5, it, :6] - base).tolist(); mm2 = (t[6, it, :3] - base).tolist()
-    print(f" it={it} tile0 [start, loop end, O ready, epilogue end, (fused split-KV: siblings arrived, merge done)] {a}  tile1 {b2}  mma [prologue, S(0) issued, loop end] {mm2}")
+    a = (t[4, it, :4] - base).tolist(); b2 = (t[5, it, :4] - base).tolist(); mm2 = (t[6, it, :3] - base).tolist()
+    print(f" it={it} tile0 [start, loop end, O ready, epilogue end] {a}  tile1 {b2}  mma [prologue, S(0) issued, loop end] {mm2}")
 if items > 2:
     per_item = np.diff(t[4, 1:items, 0]).mean()
     print(f"cycles per item {per_item:.0f}; loop {np.mean(t[4,1:items,1]-t[4,1:items,0]):.0f}; wait O {np.mean(t[4,1:items,2]-t[4,1:items,1]):.0f}; "

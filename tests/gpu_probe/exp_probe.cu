@@ -4,7 +4,7 @@
 // other tile waits for the tensor pipe) and with two (both tiles' warps in their exp phase at once).
 //   variant 0: 64 x ex2 only (the MUFU pipe's cadence as one warp sees it)
 //   variant 1: production pattern: x = s * scale - m (FFMA2), ex2 x 2, row sum (FADD2), 16-bit pack (F2FP)
-//   variant 2: same through softmax_exp_half (in place, MFA_EXP_SKEW-pipelined)
+//   variant 2: same through softmax_exp_half (in place, skewed)
 //   variant 3: x pair -> f16x2 (F2FP), ONE ex2.approx.ftz.f16x2 per pair; the result IS the packed FP16 P (no row sum:
 //              l would come from a ones column of V on the tensor core)
 //   variant 4: variant 3 plus an FP32 row sum of the unpacked results

@@ -149,7 +149,7 @@ def test_one_process_drives_two_gpus():
     if torch.cuda.device_count() < 2:
         pytest.skip("needs two GPUs in one process")
     KT = mfa.AttentionKernelType
-    for R, C, D, batch in ((256, 256, 128, 3), (4096, 4096, 128, 1)):   # plain and split-KV (fused, cooperative) grids
+    for R, C, D, batch in ((256, 256, 128, 3), (4096, 4096, 128, 1)):   # plain and split-KV grids
         desc = mfa.AttentionDescriptor()
         desc.lowPrecisionInputs = True
         desc.inputPrecisionOverride = mfa.GEMMOperandPrecision.BF16

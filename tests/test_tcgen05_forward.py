@@ -70,36 +70,28 @@ def test_forward_matches_oracle(R, C, D, bf16):
 SPLIT_KV_CASES = [(4096, 4096, 128, True),   # 16 items x 8 splits: the headline single head
                   (256, 2048, 64, False),    # 1 item x 4 splits
                   (300, 2000, 128, True),    # ragged rows and a ragged last key block
-                  (512, 1536, 96, True),     # 12 key blocks -> 3 splits: uneven row slices in the fused merge
+                  (512, 1536, 96, True),     # 12 key blocks -> 3 splits
                   (1, 4096, 128, False),     # a single query row
                   (2048, 2048, 64, True)]    # BASELINE configs[2] shape
 
 
 @pytest.mark.gpu
-@pytest.mark.parametrize("fused", [True, False], ids=["fused-one-launch", "scratch-combine"])
 @pytest.mark.parametrize("R,C,D,bf16", SPLIT_KV_CASES)
-def test_split_kv_small_grids(R, C, D, bf16, fused):
-    """Few (head, tile pair) items: the key axis is split across SMs.  Default form: normalised partials in the library's
-    workspace + the combine kernel (2 launches); one-launch form: every split CTA publishes its raw partial, waits on the
-    tile pair's arrival counter and merges a slice of the rows inside the attention kernel.  Both must match the oracle, also
-    when run back to back (the fused form must leave its counters at zero)."""
+def test_split_kv_small_grids(R, C, D, bf16):
+    """Few (head, tile pair) items: the key axis is split across SMs.  Normalised partials go to the library's workspace
+    and the combine kernel merges them (2 launches).  Must match the oracle, also when run back to back."""
     import mfa_b200 as mfa
     desc = _descriptor(R, C, D, bf16)
     kernel = mfa.AttentionKernel(desc.kernelDescriptor(mfa.AttentionKernelType.forward))
     constants = mfa.FunctionConstantValues()
     desc.setFunctionConstants(constants)
-    mfa._lib.mfa_debug_set_forward_fused(1 if fused else 0)
-    try:
-        assert kernel.launchCount(constants) == (1 if fused else 2), "split-KV should engage for this grid"
-        _run_and_check(R, C, D, bf16, seed=R + C + D)
-        _run_and_check(R, C, D, bf16, seed=R + C + D + 1)
-    finally:
-        mfa._lib.mfa_debug_set_forward_fused(0)   # library default: scratch + combine (measured faster)
+    assert kernel.launchCount(constants) == 2, "split-KV should engage for this grid"
+    _run_and_check(R, C, D, bf16, seed=R + C + D)
+    _run_and_check(R, C, D, bf16, seed=R + C + D + 1)
 
 
 @pytest.mark.gpu
-@pytest.mark.parametrize("fused", [True, False], ids=["fused-one-launch", "scratch-combine"])
-def test_split_kv_batched_heads_and_fp16_L(fused):
+def test_split_kv_batched_heads_and_fp16_L():
     """Split-KV with several heads in one launch (item -> (head, tile, split)) and FP16 L storage."""
     import mfa_b200 as mfa
     H, N, D = 3, 1024, 128
@@ -107,12 +99,8 @@ def test_split_kv_batched_heads_and_fp16_L(fused):
     kernel = mfa.AttentionKernel(desc.kernelDescriptor(mfa.AttentionKernelType.forward))
     constants = mfa.FunctionConstantValues()
     desc.setFunctionConstants(constants)
-    mfa._lib.mfa_debug_set_forward_fused(1 if fused else 0)
-    try:
-        assert kernel.launchCount(constants) == (1 if fused else 2)
-        _check_batched_cluster(desc, H, N, D)
-    finally:
-        mfa._lib.mfa_debug_set_forward_fused(0)
+    assert kernel.launchCount(constants) == 2
+    _check_batched_cluster(desc, H, N, D)
 
 
 def _check_batched_cluster(desc, H, N, D):
