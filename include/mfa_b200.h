@@ -334,6 +334,131 @@ MFA_API int mfa_release_device_resources(int device);
 MFA_API int mfa_attention_descriptor_operand_elements(const mfa_attention_descriptor_t *descriptor,
                                                       mfa_operand_t operand, size_t *out);
 
+/* ------------------------------------------------------------------------------------------ */
+/* GEMMDescriptor   (R/GEMM/GEMMDescriptor/GEMMDescriptor.swift:10-44)                          */
+/* ------------------------------------------------------------------------------------------ */
+/* C = A . B, or C += A . B with load_previous_C (AdversarialShapeTest.swift:211-236):
+ *   A is M x K (row m at m * lda), or stored K x M when transpose_A (row k at k * lda);
+ *   B is K x N (row k at k * ldb), or stored N x K when transpose_B (row n at n * ldb);
+ *   C is M x N, row-major, row m at m * ldc.
+ * Buffer bindings: A = 0, B = 1, C = 2 (GEMMKernel+Source.swift:42-44). */
+#define MFA_GEMM_BUFFER_COUNT 3
+
+typedef struct mfa_gemm_descriptor {
+  uint32_t batch_dimension;            /* batchDimension :18.  B200 extension: N > 1 runs N independent problems stored
+                                          back to back; problem b of an operand starts at b * trailing * leading
+                                          elements (trailing = rows as stored, leading = its leading dimension).  0 = 1. */
+  uint8_t has_leading_dimensions;      /* Swift optional `leadingDimensions != nil`   :21 */
+  uint8_t load_previous_C;             /* loadPreviousC                                :23 */
+  uint8_t has_matrix_dimensions;       /* Swift optional `matrixDimensions != nil`     :37 */
+  uint8_t has_memory_precisions;       /* Swift optional `memoryPrecisions != nil`     :39-40 */
+  uint8_t has_transpose_state;         /* Swift optional `transposeState != nil`       :42 */
+  uint8_t transpose_A, transpose_B;    /* transposeState (A, B) */
+  uint8_t memory_precisions[3];        /* memoryPrecisions (A, B, C), mfa_precision_t raw values */
+  uint32_t leading_dimensions[3];      /* leadingDimensions (A, B, C) */
+  uint32_t M, N, K;                    /* matrixDimensions */
+} mfa_gemm_descriptor_t;
+
+/** GEMMDescriptor.init(): batch 1, everything else nil / false. */
+MFA_API void mfa_gemm_descriptor_init(mfa_gemm_descriptor_t *descriptor);
+
+/** The launch-time constants: descriptor.setFunctionConstants(_:) (GEMMDescriptor.swift:327-380), indices 0-2 (M, N, K),
+ *  5-7 (leading dimensions) and 10 (loadPreviousC), plus the batch extension. */
+typedef struct mfa_gemm_function_constants {
+  uint32_t M, N, K;
+  uint32_t leading_dimensions[3]; /* A, B, C: the descriptor's, or the defaults of chooseLeadingDimension (:340-364) */
+  uint8_t load_previous_C;
+  uint32_t batch_count;           /* 0/1 = single problem */
+} mfa_gemm_function_constants_t;
+
+/** Fills `constants`.  Missing matrixDimensions / transposeState -> MFA_ERROR_INCOMPLETE_DESCRIPTOR ("Descriptor was
+ *  incomplete."); a leading dimension below its minimum (K or M for A, N or K for B, N for C) -> MFA_ERROR_INVALID_ARGUMENT
+ *  with "Leading block dimension was too small." (:355-357). */
+MFA_API int mfa_gemm_descriptor_set_function_constants(const mfa_gemm_descriptor_t *descriptor,
+                                                       mfa_gemm_function_constants_t *constants);
+
+/* ------------------------------------------------------------------------------------------ */
+/* GEMMKernelDescriptor   (R/GEMM/GEMMKernelDescriptor.swift:21-181)                           */
+/* ------------------------------------------------------------------------------------------ */
+typedef struct mfa_gemm_kernel_descriptor {
+  uint8_t has_block_dimensions;             /* blockDimensions (M, N, K)                       :116 */
+  uint16_t block_dimensions[3];
+  uint8_t has_leading_block_dimensions;     /* leadingBlockDimensions (A, B, C), optional      :126 */
+  uint16_t leading_block_dimensions[3];
+  uint8_t has_memory_precisions;            /* memoryPrecisions (A, B, C)                      :128 */
+  uint8_t memory_precisions[3];
+  uint8_t has_register_precisions;          /* registerPrecisions (A, B, C)                    :165 */
+  uint8_t register_precisions[3];
+  uint8_t prefer_async_load;                /* preferAsyncLoad: 0 / 1 (default 1)              :139 */
+  uint8_t prefer_async_store;               /* preferAsyncStore: 0 / 1 / 0xFF nil              :145 */
+  uint8_t has_splits;                       /* splits (M, N)                                   :173 */
+  uint16_t splits[2];
+  uint8_t has_transpose_state;              /* transposeState (A, B)                           :176 */
+  uint8_t transpose_A, transpose_B;
+  /* ---- B200 extension: which sm_100a kernel family the heuristic picked ---- */
+  uint8_t backend;                          /* mfa_backend_t */
+} mfa_gemm_kernel_descriptor_t;
+
+/** GEMMKernelDescriptor.init(): everything nil, preferAsyncLoad true. */
+MFA_API void mfa_gemm_kernel_descriptor_init(mfa_gemm_kernel_descriptor_t *kernel_descriptor);
+
+/** GEMMKernelDescriptor(descriptor:)  (GEMMDescriptor.swift:106-234), with this library's heuristic in place of the
+ *  Apple one: MFA_BACKEND_TCGEN05 when A and B are both FP16 or both BF16 (any C), MFA_BACKEND_SIMT_FP32 otherwise
+ *  (FP32 in A or B, or FP16 beside BF16: tcgen05 kind::f16 cannot mix the two 16-bit types in one MMA, and TF32 would
+ *  miss the FP32 tolerance).  Register precisions: A and B keep their memory precision; C is FP32 because both families
+ *  accumulate in FP32 (TMEM or registers) -- where the reference picks FP16 for an all-FP16 problem (:196-200).
+ *  Missing matrixDimensions / memoryPrecisions / transposeState -> MFA_ERROR_INCOMPLETE_DESCRIPTOR. */
+MFA_API int mfa_gemm_descriptor_kernel_descriptor(const mfa_gemm_descriptor_t *descriptor,
+                                                  mfa_gemm_kernel_descriptor_t *out);
+
+/* ------------------------------------------------------------------------------------------ */
+/* GEMMKernel   (R/GEMM/GEMMKernel/GEMMKernel.swift:10-270)                                     */
+/* ------------------------------------------------------------------------------------------ */
+typedef struct mfa_gemm_kernel mfa_gemm_kernel_t; /* opaque */
+
+/** GEMMKernel(descriptor:)  (:26-154).  Missing blockDimensions, memoryPrecisions, preferAsyncStore,
+ *  registerPrecisions, splits or transposeState -> MFA_ERROR_INCOMPLETE_DESCRIPTOR ("Descriptor was incomplete.").
+ *  Register precisions follow the reference's truth table (:46-97): "Operand A had an invalid register precision." (and
+ *  B, C) and "BF16 cannot be used as the register precision for C." -> MFA_ERROR_INVALID_PRECISIONS.  An FP16 register
+ *  precision for C (legal in the reference) is accepted; the kernels still accumulate in FP32.  Block or leading block
+ *  dimensions without a compiled kernel, or a backend the precisions do not fit -> MFA_ERROR_UNSUPPORTED. */
+MFA_API int mfa_gemm_kernel_create(const mfa_gemm_kernel_descriptor_t *kernel_descriptor, mfa_gemm_kernel_t **out);
+MFA_API void mfa_gemm_kernel_destroy(mfa_gemm_kernel_t *kernel);
+
+/** kernel.blockDimensions (M, N, K) of the compiled kernel  (:21). */
+MFA_API int mfa_gemm_kernel_block_dimensions(const mfa_gemm_kernel_t *kernel, uint16_t out[3]);
+/** kernel.threadgroupSize  (:260-262): threads per CTA (for tcgen05: 4 epilogue warps + 1 TMA warp + 1 MMA warp). */
+MFA_API int mfa_gemm_kernel_threadgroup_size(const mfa_gemm_kernel_t *kernel, uint32_t *out);
+/** kernel.threadgroupMemoryAllocation  (:24, 264-269): dynamic shared memory bytes per CTA. */
+MFA_API int mfa_gemm_kernel_threadgroup_memory_allocation(const mfa_gemm_kernel_t *kernel, uint32_t *out);
+/** Output tiles of the dispatch: ceil(N / block N) * ceil(M / block M) * batch (AdversarialShapeTest.swift:152-158).
+ *  The tcgen05 kernel is persistent: it launches min(tiles, SM count) CTAs that loop over these tiles. */
+MFA_API int mfa_gemm_kernel_grid_size(const mfa_gemm_kernel_t *kernel, const mfa_gemm_function_constants_t *constants,
+                                      uint32_t *out);
+/** CUDA kernels one encode() launches: 1, plus (tcgen05) one staging copy per 16-bit operand whose leading dimension is
+ *  not a multiple of 8 elements.  A base pointer that is not 16-byte aligned also stages its operand (one more launch,
+ *  which the constants alone cannot predict). */
+MFA_API int mfa_gemm_kernel_launch_count(const mfa_gemm_kernel_t *kernel, const mfa_gemm_function_constants_t *constants,
+                                         uint32_t *out);
+/** Name of the compiled kernel ("gemm_tcgen05<bfloat, bfloat, float, NN>" ...), standing in for createSource(). */
+MFA_API const char *mfa_gemm_kernel_source_name(const mfa_gemm_kernel_t *kernel);
+
+/** Binds A, B, C (device pointers, bindings 0, 1, 2) and dispatches on `cuda_stream` (NULL = default stream) of the
+ *  current device; asynchronous.  C may alias nothing else; with load_previous_C it is read and written in place.
+ *  The staging copies of the tcgen05 family use a library-owned workspace per (device, stream), which grows with
+ *  cudaMalloc: encode the same problem once outside a CUDA-graph capture before capturing it.
+ *  No sm_100 device -> MFA_ERROR_NO_DEVICE (no CPU fallback). */
+MFA_API int mfa_gemm_kernel_encode(const mfa_gemm_kernel_t *kernel, const mfa_gemm_function_constants_t *constants,
+                                   void *const buffers[MFA_GEMM_BUFFER_COUNT], void *cuda_stream);
+
+/** GEMMKernel.register(descriptor:) + pipelineCache[descriptor] (GEMMDescriptor+PipelineCache.swift:16-36): the
+ *  kernel object of the descriptor, created once.  The key is what the kernel descriptor depends on -- memory
+ *  precisions and transposes; M, N, K, the leading dimensions, load_previous_C and the batch are launch constants.  The
+ *  handle is owned by the library (do NOT destroy it), immutable and valid until process exit.  Thread-safe. */
+MFA_API int mfa_gemm_kernel_cache_fetch(const mfa_gemm_descriptor_t *descriptor, const mfa_gemm_kernel_t **out);
+/** Number of GEMM kernel objects the cache holds. */
+MFA_API int mfa_gemm_kernel_cache_size(void);
+
 #ifdef __cplusplus
 } /* extern "C" */
 #endif

@@ -14,6 +14,11 @@ reference's names, field meanings and failure behaviour:
     AttentionOperand(.bufferBinding)  Attention/AttentionOperand.swift:8-72
     AttentionKernel                Attention/AttentionKernel/AttentionKernel.swift:11-50, 268-363
     GEMMOperandPrecision           GEMM/GEMMOperandPrecision.swift:33-61
+    GEMMDescriptor                 GEMM/GEMMDescriptor/GEMMDescriptor.swift:10-44
+      .setFunctionConstants(_:)    :327-380
+    GEMMKernelDescriptor           GEMM/GEMMKernelDescriptor.swift:21-181; (descriptor:) GEMMDescriptor.swift:106-234
+    GEMMKernel                     GEMM/GEMMKernel/GEMMKernel.swift:10-270
+      .register / pipelineCache    GEMM/GEMMDescriptor/GEMMDescriptor+PipelineCache.swift:16-36
 
 All arithmetic happens in libmfa_b200.so (hand-written sm_100a CUDA).  There is no Python or CPU
 fallback: if the shared library is missing, importing this package raises.  Where the reference traps
@@ -31,6 +36,7 @@ _LIB_PATH = os.environ.get("MFA_B200_LIBRARY") or os.path.join(_HERE, "lib", "li
 
 MFA_OPERAND_COUNT = 14
 MFA_BUFFER_COUNT = 10
+MFA_GEMM_BUFFER_COUNT = 3
 
 
 class MFAError(RuntimeError):
@@ -92,6 +98,56 @@ class _CFunctionConstants(ctypes.Structure):
     _fields_ = [("row", ctypes.c_uint32), ("column", ctypes.c_uint32), ("batch_count", ctypes.c_uint32)]
 
 
+class _CGEMMDescriptor(ctypes.Structure):
+    _fields_ = [
+        ("batch_dimension", ctypes.c_uint32),
+        ("has_leading_dimensions", ctypes.c_uint8),
+        ("load_previous_C", ctypes.c_uint8),
+        ("has_matrix_dimensions", ctypes.c_uint8),
+        ("has_memory_precisions", ctypes.c_uint8),
+        ("has_transpose_state", ctypes.c_uint8),
+        ("transpose_A", ctypes.c_uint8),
+        ("transpose_B", ctypes.c_uint8),
+        ("memory_precisions", ctypes.c_uint8 * 3),
+        ("leading_dimensions", ctypes.c_uint32 * 3),
+        ("M", ctypes.c_uint32),
+        ("N", ctypes.c_uint32),
+        ("K", ctypes.c_uint32),
+    ]
+
+
+class _CGEMMFunctionConstants(ctypes.Structure):
+    _fields_ = [
+        ("M", ctypes.c_uint32),
+        ("N", ctypes.c_uint32),
+        ("K", ctypes.c_uint32),
+        ("leading_dimensions", ctypes.c_uint32 * 3),
+        ("load_previous_C", ctypes.c_uint8),
+        ("batch_count", ctypes.c_uint32),
+    ]
+
+
+class _CGEMMKernelDescriptor(ctypes.Structure):
+    _fields_ = [
+        ("has_block_dimensions", ctypes.c_uint8),
+        ("block_dimensions", ctypes.c_uint16 * 3),
+        ("has_leading_block_dimensions", ctypes.c_uint8),
+        ("leading_block_dimensions", ctypes.c_uint16 * 3),
+        ("has_memory_precisions", ctypes.c_uint8),
+        ("memory_precisions", ctypes.c_uint8 * 3),
+        ("has_register_precisions", ctypes.c_uint8),
+        ("register_precisions", ctypes.c_uint8 * 3),
+        ("prefer_async_load", ctypes.c_uint8),
+        ("prefer_async_store", ctypes.c_uint8),
+        ("has_splits", ctypes.c_uint8),
+        ("splits", ctypes.c_uint16 * 2),
+        ("has_transpose_state", ctypes.c_uint8),
+        ("transpose_A", ctypes.c_uint8),
+        ("transpose_B", ctypes.c_uint8),
+        ("backend", ctypes.c_uint8),
+    ]
+
+
 def _load():
     if not os.path.exists(_LIB_PATH):
         raise ImportError(
@@ -131,6 +187,27 @@ def _load():
     lib.mfa_attention_kernel_cache_size.restype = c.c_int
     lib.mfa_attention_run_host.argtypes = [c.POINTER(_CDescriptor), c.c_uint32,
                                            c.POINTER(c.c_void_p * MFA_BUFFER_COUNT), c.c_int]
+    lib.mfa_gemm_descriptor_init.argtypes = [c.POINTER(_CGEMMDescriptor)]
+    lib.mfa_gemm_descriptor_init.restype = None
+    lib.mfa_gemm_descriptor_set_function_constants.argtypes = [c.POINTER(_CGEMMDescriptor),
+                                                               c.POINTER(_CGEMMFunctionConstants)]
+    lib.mfa_gemm_kernel_descriptor_init.argtypes = [c.POINTER(_CGEMMKernelDescriptor)]
+    lib.mfa_gemm_kernel_descriptor_init.restype = None
+    lib.mfa_gemm_descriptor_kernel_descriptor.argtypes = [c.POINTER(_CGEMMDescriptor), c.POINTER(_CGEMMKernelDescriptor)]
+    lib.mfa_gemm_kernel_create.argtypes = [c.POINTER(_CGEMMKernelDescriptor), c.POINTER(c.c_void_p)]
+    lib.mfa_gemm_kernel_destroy.argtypes = [c.c_void_p]
+    lib.mfa_gemm_kernel_destroy.restype = None
+    lib.mfa_gemm_kernel_block_dimensions.argtypes = [c.c_void_p, c.POINTER(c.c_uint16 * 3)]
+    lib.mfa_gemm_kernel_threadgroup_size.argtypes = [c.c_void_p, c.POINTER(c.c_uint32)]
+    lib.mfa_gemm_kernel_threadgroup_memory_allocation.argtypes = [c.c_void_p, c.POINTER(c.c_uint32)]
+    lib.mfa_gemm_kernel_grid_size.argtypes = [c.c_void_p, c.POINTER(_CGEMMFunctionConstants), c.POINTER(c.c_uint32)]
+    lib.mfa_gemm_kernel_launch_count.argtypes = [c.c_void_p, c.POINTER(_CGEMMFunctionConstants), c.POINTER(c.c_uint32)]
+    lib.mfa_gemm_kernel_source_name.argtypes = [c.c_void_p]
+    lib.mfa_gemm_kernel_source_name.restype = c.c_char_p
+    lib.mfa_gemm_kernel_encode.argtypes = [c.c_void_p, c.POINTER(_CGEMMFunctionConstants),
+                                           c.POINTER(c.c_void_p * MFA_GEMM_BUFFER_COUNT), c.c_void_p]
+    lib.mfa_gemm_kernel_cache_fetch.argtypes = [c.POINTER(_CGEMMDescriptor), c.POINTER(c.c_void_p)]
+    lib.mfa_gemm_kernel_cache_size.restype = c.c_int
     try:
         lib.mfa_set_parameter_table.argtypes = [c.c_int, c.c_int, c.c_char_p]
         lib.mfa_host_alloc.argtypes = [c.c_size_t, c.c_int, c.POINTER(c.c_void_p)]
@@ -538,7 +615,254 @@ class AttentionKernel:
                                                 ctypes.c_void_p(stream)))
 
 
+# -------------------------------------------------------------------------------------------------
+# GEMM: GEMMDescriptor, GEMMKernelDescriptor, GEMMKernel
+# -------------------------------------------------------------------------------------------------
+def _triple(values, cast=int):
+    return tuple(cast(v) for v in values)
+
+
+class GEMMDescriptor:
+    """GEMMDescriptor.swift:10-44.  C = A . B (or C += A . B with loadPreviousC).  `matrixDimensions = (M, N, K)`,
+    `memoryPrecisions = (A, B, C)`, `transposeState = (A, B)`, `leadingDimensions = (A, B, C)`; the optionals start as
+    None.  batchDimension > 1 (B200 extension): independent problems stored back to back."""
+
+    def __init__(self):
+        self.batchDimension: int = 1
+        self.leadingDimensions: Optional[Tuple[int, int, int]] = None
+        self.loadPreviousC: bool = False
+        self.matrixDimensions: Optional[Tuple[int, int, int]] = None
+        self.memoryPrecisions: Optional[Tuple[GEMMOperandPrecision, GEMMOperandPrecision, GEMMOperandPrecision]] = None
+        self.transposeState: Optional[Tuple[bool, bool]] = None
+
+    def _c(self) -> _CGEMMDescriptor:
+        d = _CGEMMDescriptor()
+        _lib.mfa_gemm_descriptor_init(ctypes.byref(d))
+        d.batch_dimension = int(self.batchDimension)
+        if self.leadingDimensions is not None:
+            d.has_leading_dimensions = 1
+            d.leading_dimensions[:] = _triple(self.leadingDimensions)
+        d.load_previous_C = int(bool(self.loadPreviousC))
+        if self.matrixDimensions is not None:
+            d.has_matrix_dimensions = 1
+            d.M, d.N, d.K = _triple(self.matrixDimensions)
+        if self.memoryPrecisions is not None:
+            d.has_memory_precisions = 1
+            d.memory_precisions[:] = _triple(self.memoryPrecisions)
+        if self.transposeState is not None:
+            d.has_transpose_state = 1
+            d.transpose_A, d.transpose_B = (int(bool(x)) for x in self.transposeState)
+        return d
+
+    def setFunctionConstants(self, constants: "GEMMFunctionConstantValues") -> None:
+        """M, N, K, the leading dimensions (chooseLeadingDimension's defaults when None), loadPreviousC, the batch."""
+        c = self._c()
+        _check(_lib.mfa_gemm_descriptor_set_function_constants(ctypes.byref(c), ctypes.byref(constants._c)))
+
+
+class GEMMFunctionConstantValues:
+    """Stand-in for the MTLFunctionConstantValues GEMMDescriptor.setFunctionConstants fills (indices 0-2, 5-7, 10)."""
+
+    def __init__(self):
+        self._c = _CGEMMFunctionConstants()
+
+    @property
+    def matrixDimensions(self) -> Tuple[int, int, int]:
+        return (self._c.M, self._c.N, self._c.K)
+
+    @property
+    def leadingDimensions(self) -> Tuple[int, int, int]:
+        return tuple(self._c.leading_dimensions)
+
+    @property
+    def loadPreviousC(self) -> bool:
+        return bool(self._c.load_previous_C)
+
+    @property
+    def batchCount(self) -> int:
+        return self._c.batch_count
+
+
+class GEMMKernelDescriptor:
+    """GEMMKernelDescriptor.swift:21-181 (a plain, editable value).  GEMMKernelDescriptor(descriptor) runs this
+    library's heuristic (GEMMDescriptor.swift:106-234 analogue); GEMMKernelDescriptor() is the empty one."""
+
+    def __init__(self, descriptor: Optional[GEMMDescriptor] = None):
+        self._c = _CGEMMKernelDescriptor()
+        _lib.mfa_gemm_kernel_descriptor_init(ctypes.byref(self._c))
+        if descriptor is not None:
+            d = descriptor._c()
+            _check(_lib.mfa_gemm_descriptor_kernel_descriptor(ctypes.byref(d), ctypes.byref(self._c)))
+
+    def _get3(self, flag, array, cast=int):
+        return tuple(cast(v) for v in array) if getattr(self._c, flag) else None
+
+    def _set3(self, flag, name, value):
+        if value is None:
+            setattr(self._c, flag, 0)
+        else:
+            setattr(self._c, flag, 1)
+            getattr(self._c, name)[:] = _triple(value)
+
+    @property
+    def blockDimensions(self) -> Optional[Tuple[int, int, int]]:
+        return self._get3("has_block_dimensions", self._c.block_dimensions)
+
+    @blockDimensions.setter
+    def blockDimensions(self, value):
+        self._set3("has_block_dimensions", "block_dimensions", value)
+
+    @property
+    def leadingBlockDimensions(self) -> Optional[Tuple[int, int, int]]:
+        return self._get3("has_leading_block_dimensions", self._c.leading_block_dimensions)
+
+    @leadingBlockDimensions.setter
+    def leadingBlockDimensions(self, value):
+        self._set3("has_leading_block_dimensions", "leading_block_dimensions", value)
+
+    @property
+    def memoryPrecisions(self):
+        return self._get3("has_memory_precisions", self._c.memory_precisions, GEMMOperandPrecision)
+
+    @memoryPrecisions.setter
+    def memoryPrecisions(self, value):
+        self._set3("has_memory_precisions", "memory_precisions", value)
+
+    @property
+    def registerPrecisions(self):
+        return self._get3("has_register_precisions", self._c.register_precisions, GEMMOperandPrecision)
+
+    @registerPrecisions.setter
+    def registerPrecisions(self, value):
+        self._set3("has_register_precisions", "register_precisions", value)
+
+    @property
+    def preferAsyncLoad(self) -> bool:
+        return bool(self._c.prefer_async_load)
+
+    @preferAsyncLoad.setter
+    def preferAsyncLoad(self, value):
+        self._c.prefer_async_load = int(bool(value))
+
+    @property
+    def preferAsyncStore(self) -> Optional[bool]:
+        return None if self._c.prefer_async_store == 0xFF else bool(self._c.prefer_async_store)
+
+    @preferAsyncStore.setter
+    def preferAsyncStore(self, value):
+        self._c.prefer_async_store = 0xFF if value is None else int(bool(value))
+
+    @property
+    def splits(self) -> Optional[Tuple[int, int]]:
+        return (self._c.splits[0], self._c.splits[1]) if self._c.has_splits else None
+
+    @splits.setter
+    def splits(self, value):
+        if value is None:
+            self._c.has_splits = 0
+        else:
+            self._c.has_splits = 1
+            self._c.splits[0], self._c.splits[1] = (int(v) for v in value)
+
+    @property
+    def transposeState(self) -> Optional[Tuple[bool, bool]]:
+        return (bool(self._c.transpose_A), bool(self._c.transpose_B)) if self._c.has_transpose_state else None
+
+    @transposeState.setter
+    def transposeState(self, value):
+        if value is None:
+            self._c.has_transpose_state = 0
+        else:
+            self._c.has_transpose_state = 1
+            self._c.transpose_A, self._c.transpose_B = (int(bool(v)) for v in value)
+
+    @property
+    def backend(self) -> Backend:
+        return Backend(self._c.backend)
+
+    @backend.setter
+    def backend(self, value):
+        self._c.backend = int(value)
+
+
+class GEMMKernel:
+    """GEMMKernel.swift:10-270.  `encode` binds A, B, C (device pointers, bindings 0, 1, 2) and dispatches, which the
+    reference leaves to its caller (AdversarialShapeTest.swift:140-169)."""
+
+    def __init__(self, descriptor: GEMMKernelDescriptor):
+        self._handle = ctypes.c_void_p()
+        self._owned = True
+        _check(_lib.mfa_gemm_kernel_create(ctypes.byref(descriptor._c), ctypes.byref(self._handle)))
+
+    @classmethod
+    def register(cls, descriptor: GEMMDescriptor) -> None:
+        """GEMMKernel.register(descriptor:): build the descriptor's kernel object once (GEMMDescriptor+PipelineCache.swift:
+        24-36)."""
+        cls.cached(descriptor)
+
+    @classmethod
+    def cached(cls, descriptor: GEMMDescriptor) -> "GEMMKernel":
+        """pipelineCache[descriptor]: the library-owned kernel object (mfa_gemm_kernel_cache_fetch).  The key is the
+        precisions and transposes; M, N, K, leading dimensions, loadPreviousC and the batch are launch constants."""
+        self = cls.__new__(cls)
+        self._handle = ctypes.c_void_p()
+        self._owned = False
+        c = descriptor._c()
+        _check(_lib.mfa_gemm_kernel_cache_fetch(ctypes.byref(c), ctypes.byref(self._handle)))
+        return self
+
+    @staticmethod
+    def cacheSize() -> int:
+        return _lib.mfa_gemm_kernel_cache_size()
+
+    def __del__(self):
+        handle = getattr(self, "_handle", None)
+        if handle and getattr(self, "_owned", False) and _lib is not None:
+            _lib.mfa_gemm_kernel_destroy(handle)
+            self._handle = None
+
+    @property
+    def blockDimensions(self) -> Tuple[int, int, int]:
+        out = (ctypes.c_uint16 * 3)()
+        _check(_lib.mfa_gemm_kernel_block_dimensions(self._handle, ctypes.byref(out)))
+        return (out[0], out[1], out[2])
+
+    @property
+    def threadgroupSize(self) -> int:
+        out = ctypes.c_uint32()
+        _check(_lib.mfa_gemm_kernel_threadgroup_size(self._handle, ctypes.byref(out)))
+        return out.value
+
+    @property
+    def threadgroupMemoryAllocation(self) -> int:
+        out = ctypes.c_uint32()
+        _check(_lib.mfa_gemm_kernel_threadgroup_memory_allocation(self._handle, ctypes.byref(out)))
+        return out.value
+
+    def gridSize(self, constants: GEMMFunctionConstantValues) -> int:
+        out = ctypes.c_uint32()
+        _check(_lib.mfa_gemm_kernel_grid_size(self._handle, ctypes.byref(constants._c), ctypes.byref(out)))
+        return out.value
+
+    def launchCount(self, constants: GEMMFunctionConstantValues) -> int:
+        out = ctypes.c_uint32()
+        _check(_lib.mfa_gemm_kernel_launch_count(self._handle, ctypes.byref(constants._c), ctypes.byref(out)))
+        return out.value
+
+    def sourceName(self) -> str:
+        return _lib.mfa_gemm_kernel_source_name(self._handle).decode()
+
+    def encode(self, constants: GEMMFunctionConstantValues, buffers: Sequence[int], stream: int = 0) -> None:
+        """buffers: device pointers of (A, B, C); stream: cudaStream_t as int (0 = default)."""
+        if len(buffers) != MFA_GEMM_BUFFER_COUNT:
+            raise MFAError(-2, "GEMM encode takes three buffers: A, B, C.")
+        arr = (ctypes.c_void_p * MFA_GEMM_BUFFER_COUNT)(*buffers)
+        _check(_lib.mfa_gemm_kernel_encode(self._handle, ctypes.byref(constants._c), ctypes.byref(arr),
+                                           ctypes.c_void_p(stream)))
+
+
 __all__ = [
+    "GEMMDescriptor", "GEMMFunctionConstantValues", "GEMMKernelDescriptor", "GEMMKernel",
     "AttentionDescriptor", "AttentionKernelDescriptor", "AttentionKernel", "AttentionKernelType",
     "AttentionOperand", "GEMMOperandPrecision", "FunctionConstantValues", "Backend", "MFAError",
     "library_path", "version", "setParameterTable", "maxExp2FmaQuarters", "hostAlloc", "hostFree", "bindThreadToDevice", "releaseDeviceResources",

@@ -69,7 +69,7 @@ static const int *operands_of(int type, int *count) {
 
 // sm_100 check of the current device, cached per device ordinal (encode() of a microsecond-scale kernel must not pay
 // two runtime queries per call)
-static int check_device() {
+int check_device() {
   const int device = current_device();
   if (device < 0)
     return fail(MFA_ERROR_NO_DEVICE, "No CUDA device (cudaGetDevice failed; this library has no CPU fallback).");

@@ -26,7 +26,9 @@ cudaError_t ensure_max_dynamic_smem(const void *kernel, uint32_t bytes, int devi
 // needs more room.  The block is cudaMalloc-aligned (256 B), which the tensor map over the forward's split partials needs.
 // `slot` separates independent users inside one encode(): 0 = split partials (forward / backward launchers), 1 = the
 // head-dimension padding staging of kernel.cpp, which is live across the launcher's own use of slot 0, 2 = the FP16
-// copy of a BF16 dO (backward launchers), which is live across their use of slot 0.
+// copy of a BF16 dO (backward launchers), which is live across their use of slot 0, 3 = the zero-padded staging copies
+// of GEMM operands TMA cannot address in place (tcgen05_gemm.cu: leading dimension not a multiple of 8 elements, or a
+// base that is not 16-byte aligned).
 cudaError_t workspace_for(int device, cudaStream_t stream, size_t bytes, void **out, int slot = 0);
 
 // Frees every workspace of `device` (the device must be idle); used by tests and by mfa_release_device_resources().

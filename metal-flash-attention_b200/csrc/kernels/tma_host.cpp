@@ -46,9 +46,10 @@ namespace {
 struct MapKey {
   const void *base;
   uint32_t seq, D, batch, boxCols, boxRows, dtype;
+  uint64_t rowPitch, batchStride;  // bytes
   bool operator==(const MapKey &o) const {
     return base == o.base && seq == o.seq && D == o.D && batch == o.batch && boxCols == o.boxCols &&
-           boxRows == o.boxRows && dtype == o.dtype;
+           boxRows == o.boxRows && dtype == o.dtype && rowPitch == o.rowPitch && batchStride == o.batchStride;
   }
 };
 struct MapEntry {
@@ -62,13 +63,16 @@ uint32_t map_slot(const MapKey &k) {
   uint64_t h = reinterpret_cast<uintptr_t>(k.base) * 0x9E3779B97F4A7C15ull;
   h ^= (static_cast<uint64_t>(k.seq) << 32 | k.D) * 0xC2B2AE3D27D4EB4Full;
   h ^= (static_cast<uint64_t>(k.batch) << 32 | (k.boxRows << 8) | k.dtype) * 0x165667B19E3779F9ull;
+  h ^= (k.rowPitch ^ (k.batchStride << 20)) * 0x27D4EB2F165667C5ull;
   return static_cast<uint32_t>(h >> 40) % kMapCacheEntries;
 }
 }  // namespace
 
-static cudaError_t encode(CUtensorMap *map, CUtensorMapDataType dtype, uint32_t elemBytes, const void *base,
-                          uint32_t seq, uint32_t D, uint32_t batch, uint32_t boxCols, uint32_t boxRows) {
-  const MapKey key{base, seq, D, batch, boxCols, boxRows, static_cast<uint32_t>(dtype)};
+// [batch][seq][D] with rows rowPitch bytes apart and problems batchStride bytes apart, boxes of boxCols x boxRows x 1
+static cudaError_t encode_strided(CUtensorMap *map, CUtensorMapDataType dtype, uint32_t elemBytes, const void *base,
+                                  uint32_t seq, uint32_t D, uint32_t batch, uint64_t rowPitch, uint64_t batchStride,
+                                  uint32_t boxCols, uint32_t boxRows) {
+  const MapKey key{base, seq, D, batch, boxCols, boxRows, static_cast<uint32_t>(dtype), rowPitch, batchStride};
   MapEntry &entry = g_map_cache[map_slot(key)];
   if (entry.valid && entry.key == key) {
     *map = entry.map;
@@ -79,12 +83,13 @@ static cudaError_t encode(CUtensorMap *map, CUtensorMapDataType dtype, uint32_t 
     set_launch_detail("cuTensorMapEncodeTiled is not available from this driver");
     return cudaErrorNotSupported;
   }
-  if (reinterpret_cast<uintptr_t>(base) % 16 != 0 || (static_cast<uint64_t>(D) * elemBytes) % 16 != 0) {
-    set_launch_detail("TMA needs 16-byte aligned buffers and row pitch (base=%p, D=%u)", base, D);
+  if (reinterpret_cast<uintptr_t>(base) % 16 != 0 || rowPitch % 16 != 0 || batchStride % 16 != 0) {
+    set_launch_detail("TMA needs 16-byte aligned buffers and row pitch (base=%p, D=%u, pitch=%llu B)", base, D,
+                      (unsigned long long)rowPitch);
     return cudaErrorInvalidValue;
   }
   cuuint64_t dims[3] = {D, seq, batch};
-  cuuint64_t strides[2] = {static_cast<cuuint64_t>(D) * elemBytes, static_cast<cuuint64_t>(seq) * D * elemBytes};
+  cuuint64_t strides[2] = {rowPitch, batchStride};
   cuuint32_t box[3] = {boxCols, boxRows, 1};
   cuuint32_t elemStrides[3] = {1, 1, 1};
   CUresult r = fn(map, dtype, 3, const_cast<void *>(base), dims, strides, box, elemStrides, CU_TENSOR_MAP_INTERLEAVE_NONE,
@@ -98,6 +103,13 @@ static cudaError_t encode(CUtensorMap *map, CUtensorMapDataType dtype, uint32_t 
   entry.map = *map;
   entry.valid = true;
   return cudaSuccess;
+}
+
+// contiguous rows of D elements and contiguous problems: what every attention operand is
+static cudaError_t encode(CUtensorMap *map, CUtensorMapDataType dtype, uint32_t elemBytes, const void *base,
+                          uint32_t seq, uint32_t D, uint32_t batch, uint32_t boxCols, uint32_t boxRows) {
+  const uint64_t pitch = static_cast<uint64_t>(D) * elemBytes;
+  return encode_strided(map, dtype, elemBytes, base, seq, D, batch, pitch, pitch * seq, boxCols, boxRows);
 }
 
 cudaError_t make_tensor_map_16bit(CUtensorMap *map, const void *base, uint32_t seq, uint32_t D, uint32_t batch,
@@ -116,6 +128,13 @@ cudaError_t make_tensor_map_16bit_transposed(CUtensorMap *map, const void *base,
 cudaError_t make_tensor_map_f32(CUtensorMap *map, const void *base, uint32_t seq, uint32_t D, uint32_t batch,
                                 uint32_t box_rows) {
   return encode(map, CU_TENSOR_MAP_DATA_TYPE_FLOAT32, 4, base, seq, D, batch, 32, box_rows);
+}
+
+cudaError_t make_tensor_map_16bit_strided(CUtensorMap *map, const void *base, uint32_t rows, uint32_t cols,
+                                          uint32_t batch, uint64_t row_pitch, uint64_t batch_stride, uint32_t box_cols,
+                                          uint32_t box_rows) {
+  return encode_strided(map, CU_TENSOR_MAP_DATA_TYPE_BFLOAT16, 2, base, rows, cols, batch, row_pitch * 2,
+                        batch_stride * 2, box_cols, box_rows);
 }
 
 }  // namespace mfa

@@ -22,6 +22,14 @@ cudaError_t make_tensor_map_16bit_transposed(CUtensorMap *map, const void *base,
 cudaError_t make_tensor_map_f32(CUtensorMap *map, const void *base, uint32_t seq, uint32_t D, uint32_t batch,
                                 uint32_t box_rows);
 
+// A [batch][rows][cols] matrix of 16-bit elements whose rows are `row_pitch` elements apart and whose problems are
+// `batch_stride` elements apart (a GEMM operand with a leading dimension larger than its width), tiled as boxes of
+// box_cols x box_rows x 1 with 128-byte swizzle; elements beyond `cols` or `rows` read as zero.  The pitch and the
+// stride must be multiples of 8 elements and the base 16-byte aligned.
+cudaError_t make_tensor_map_16bit_strided(CUtensorMap *map, const void *base, uint32_t rows, uint32_t cols,
+                                          uint32_t batch, uint64_t row_pitch, uint64_t batch_stride, uint32_t box_cols,
+                                          uint32_t box_rows);
+
 void set_launch_detail(const char *fmt, ...);
 
 }  // namespace mfa

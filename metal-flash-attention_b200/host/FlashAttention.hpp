@@ -1,8 +1,8 @@
 // FlashAttention.hpp -- header-only C++ mirror of the reference's Swift value types over the C ABI
 // (include/mfa_b200.h).  The reference is compiled Swift; Swift is not installed in this image, so this is the
 // compiled-language host layer "above the C ABI": same type and member names as
-// Sources/FlashAttention/Attention/{AttentionDescriptor,AttentionKernelDescriptor,AttentionKernel}.swift,
-// same validation, and fatalError() behaviour surfaced as std::runtime_error carrying the reference's message.
+// Sources/FlashAttention/Attention/{AttentionDescriptor,AttentionKernelDescriptor,AttentionKernel}.swift and
+// Sources/FlashAttention/GEMM/{GEMMDescriptor,GEMMKernelDescriptor,GEMMKernel}.swift, same validation, and fatalError() behaviour surfaced as std::runtime_error carrying the reference's message.
 #pragma once
 #include <array>
 #include <optional>
@@ -148,6 +148,112 @@ class AttentionKernel {  // AttentionKernel.swift:11-50
   }
  private:
   mfa_attention_kernel_t *handle_ = nullptr;
+  bool owned_ = true;
+};
+
+// ------------------------------------------------------------------------------------------------------------------
+// GEMM (Sources/FlashAttention/GEMM/): C = A . B, or C += A . B with loadPreviousC
+// ------------------------------------------------------------------------------------------------------------------
+struct GEMMMatrixDimensions { uint32_t M, N, K; };
+struct GEMMLeadingDimensions { uint32_t A, B, C; };
+struct GEMMPrecisions { GEMMOperandPrecision A, B, C; };
+struct GEMMTransposeState { bool A, B; };
+
+struct GEMMDescriptor {  // GEMMDescriptor.swift:10-44
+  uint32_t batchDimension = 1;  // > 1: B200 extension, independent problems stored back to back
+  std::optional<GEMMLeadingDimensions> leadingDimensions;
+  bool loadPreviousC = false;
+  std::optional<GEMMMatrixDimensions> matrixDimensions;
+  std::optional<GEMMPrecisions> memoryPrecisions;
+  std::optional<GEMMTransposeState> transposeState;
+
+  mfa_gemm_descriptor_t c() const {
+    mfa_gemm_descriptor_t d;
+    mfa_gemm_descriptor_init(&d);
+    d.batch_dimension = batchDimension;
+    if (leadingDimensions) {
+      d.has_leading_dimensions = 1;
+      d.leading_dimensions[0] = leadingDimensions->A;
+      d.leading_dimensions[1] = leadingDimensions->B;
+      d.leading_dimensions[2] = leadingDimensions->C;
+    }
+    d.load_previous_C = loadPreviousC;
+    if (matrixDimensions) {
+      d.has_matrix_dimensions = 1;
+      d.M = matrixDimensions->M; d.N = matrixDimensions->N; d.K = matrixDimensions->K;
+    }
+    if (memoryPrecisions) {
+      d.has_memory_precisions = 1;
+      d.memory_precisions[0] = static_cast<uint8_t>(memoryPrecisions->A);
+      d.memory_precisions[1] = static_cast<uint8_t>(memoryPrecisions->B);
+      d.memory_precisions[2] = static_cast<uint8_t>(memoryPrecisions->C);
+    }
+    if (transposeState) {
+      d.has_transpose_state = 1;
+      d.transpose_A = transposeState->A; d.transpose_B = transposeState->B;
+    }
+    return d;
+  }
+  void setFunctionConstants(mfa_gemm_function_constants_t &constants) const {  // GEMMDescriptor.swift:327-380
+    mfa_gemm_descriptor_t d = c();
+    check(mfa_gemm_descriptor_set_function_constants(&d, &constants));
+  }
+};
+
+struct GEMMKernelDescriptor {  // GEMMKernelDescriptor.swift:21-181; the raw fields stay editable through `c`
+  mfa_gemm_kernel_descriptor_t c;
+  GEMMKernelDescriptor() { mfa_gemm_kernel_descriptor_init(&c); }
+  explicit GEMMKernelDescriptor(const GEMMDescriptor &descriptor) {  // GEMMDescriptor.swift:106-234
+    mfa_gemm_descriptor_t d = descriptor.c();
+    check(mfa_gemm_descriptor_kernel_descriptor(&d, &c));
+  }
+  std::optional<std::tuple<uint16_t, uint16_t, uint16_t>> blockDimensions() const {
+    if (!c.has_block_dimensions) return std::nullopt;
+    return std::make_tuple(c.block_dimensions[0], c.block_dimensions[1], c.block_dimensions[2]);
+  }
+  bool tensorCoreFamily() const { return c.backend == MFA_BACKEND_TCGEN05; }
+};
+
+class GEMMKernel {  // GEMMKernel.swift:10-270
+ public:
+  explicit GEMMKernel(const GEMMKernelDescriptor &descriptor) { check(mfa_gemm_kernel_create(&descriptor.c, &handle_)); }
+  // GEMMKernel.register(descriptor:) + pipelineCache[descriptor] (GEMMDescriptor+PipelineCache.swift:16-36): the
+  // library-owned kernel object of the descriptor (`register` is a C++ keyword, hence the underscore)
+  static void register_(const GEMMDescriptor &descriptor) { GEMMKernel unused(descriptor); }
+  static GEMMKernel cached(const GEMMDescriptor &descriptor) { return GEMMKernel(descriptor); }
+  explicit GEMMKernel(const GEMMDescriptor &descriptor) : owned_(false) {
+    mfa_gemm_descriptor_t d = descriptor.c();
+    const mfa_gemm_kernel_t *out = nullptr;
+    check(mfa_gemm_kernel_cache_fetch(&d, &out));
+    handle_ = const_cast<mfa_gemm_kernel_t *>(out);
+  }
+  static int cacheSize() { return mfa_gemm_kernel_cache_size(); }
+  ~GEMMKernel() { if (owned_) mfa_gemm_kernel_destroy(handle_); }
+  GEMMKernel(const GEMMKernel &) = delete;
+  GEMMKernel &operator=(const GEMMKernel &) = delete;
+  std::tuple<uint16_t, uint16_t, uint16_t> blockDimensions() const {
+    uint16_t out[3];
+    check(mfa_gemm_kernel_block_dimensions(handle_, out));
+    return {out[0], out[1], out[2]};
+  }
+  uint32_t threadgroupSize() const { uint32_t v; check(mfa_gemm_kernel_threadgroup_size(handle_, &v)); return v; }
+  uint32_t threadgroupMemoryAllocation() const {
+    uint32_t v; check(mfa_gemm_kernel_threadgroup_memory_allocation(handle_, &v)); return v;
+  }
+  uint32_t gridSize(const mfa_gemm_function_constants_t &constants) const {
+    uint32_t v; check(mfa_gemm_kernel_grid_size(handle_, &constants, &v)); return v;
+  }
+  uint32_t launchCount(const mfa_gemm_function_constants_t &constants) const {
+    uint32_t v; check(mfa_gemm_kernel_launch_count(handle_, &constants, &v)); return v;
+  }
+  std::string sourceName() const { return mfa_gemm_kernel_source_name(handle_); }
+  // bind A, B, C (device pointers, bindings 0, 1, 2; GEMMKernel+Source.swift:42-44) + dispatch
+  void encode(const mfa_gemm_function_constants_t &constants, const std::array<void *, MFA_GEMM_BUFFER_COUNT> &buffers,
+              void *cudaStream = nullptr) const {
+    check(mfa_gemm_kernel_encode(handle_, &constants, buffers.data(), cudaStream));
+  }
+ private:
+  mfa_gemm_kernel_t *handle_ = nullptr;
   bool owned_ = true;
 };
 

@@ -2,7 +2,8 @@
 //  FlashAttention.swift -- drop-in Swift surface over the B200 C ABI.
 //
 //  Same public names, fields and failure behaviour as the reference package
-//  (Sources/FlashAttention/Attention/*.swift), minus everything Metal-specific:
+//  (Sources/FlashAttention/Attention/*.swift, Sources/FlashAttention/GEMM/*.swift), minus everything
+//  Metal-specific:
 //    * `createSource()` is replaced by `encode(...)`: the kernels are ahead-of-time compiled CUDA, so
 //      the compile + bind + dispatch the reference leaves to its caller happens behind the C ABI.
 //    * `setFunctionConstants(_:)` fills a plain struct instead of MTLFunctionConstantValues.
@@ -376,5 +377,206 @@ public final class AttentionKernel {
     }
     var constants = constants
     check(mfa_attention_kernel_encode(handle, &constants, &table, stream))
+  }
+}
+
+// MARK: - GEMM (Sources/FlashAttention/GEMM/): C = A . B, or C += A . B with loadPreviousC
+
+/// GEMMDescriptor.swift:10-44
+public struct GEMMDescriptor: Hashable {
+  /// B200 extension beyond the block-size heuristic: N > 1 runs N problems stored back to back.
+  public var batchDimension: Int = 1
+  public var leadingDimensions: (A: UInt32, B: UInt32, C: UInt32)?
+  public var loadPreviousC: Bool = false
+  public var matrixDimensions: (M: UInt32, N: UInt32, K: UInt32)?
+  public var memoryPrecisions: (A: GEMMOperandPrecision, B: GEMMOperandPrecision, C: GEMMOperandPrecision)?
+  public var transposeState: (A: Bool, B: Bool)?
+
+  public init() {}
+
+  var c: mfa_gemm_descriptor_t {
+    var d = mfa_gemm_descriptor_t()
+    mfa_gemm_descriptor_init(&d)
+    d.batch_dimension = UInt32(batchDimension)
+    if let l = leadingDimensions {
+      d.has_leading_dimensions = 1
+      d.leading_dimensions = (l.A, l.B, l.C)
+    }
+    d.load_previous_C = loadPreviousC ? 1 : 0
+    if let m = matrixDimensions {
+      d.has_matrix_dimensions = 1
+      d.M = m.M; d.N = m.N; d.K = m.K
+    }
+    if let p = memoryPrecisions {
+      d.has_memory_precisions = 1
+      d.memory_precisions = (UInt8(p.A.rawValue), UInt8(p.B.rawValue), UInt8(p.C.rawValue))
+    }
+    if let t = transposeState {
+      d.has_transpose_state = 1
+      d.transpose_A = t.A ? 1 : 0; d.transpose_B = t.B ? 1 : 0
+    }
+    return d
+  }
+
+  /// GEMMDescriptor.swift:327-380: M, N, K, the leading dimensions (chooseLeadingDimension's defaults when nil),
+  /// loadPreviousC and the batch, into a plain struct instead of MTLFunctionConstantValues.
+  public func setFunctionConstants(_ constants: inout mfa_gemm_function_constants_t) {
+    var d = c
+    check(mfa_gemm_descriptor_set_function_constants(&d, &constants))
+  }
+
+  // Equal when GEMMKey (GEMMDescriptor.swift:49-90) is: the C struct is compared field by field.
+  public static func == (lhs: GEMMDescriptor, rhs: GEMMDescriptor) -> Bool {
+    let l = lhs.c, r = rhs.c
+    return withUnsafeBytes(of: l) { a in withUnsafeBytes(of: r) { b in a.elementsEqual(b) } }
+  }
+  public func hash(into hasher: inout Hasher) {
+    withUnsafeBytes(of: c) { hasher.combine(bytes: $0) }
+  }
+}
+
+/// GEMMKernelDescriptor.swift:21-181 -- a plain, editable value; storage is the C struct.
+public struct GEMMKernelDescriptor {
+  public var c = mfa_gemm_kernel_descriptor_t()
+  public init() { mfa_gemm_kernel_descriptor_init(&c) }
+  /// GEMMDescriptor.swift:106-234, with this library's heuristic: the tcgen05 family when A and B are both FP16 or
+  /// both BF16, the SIMT FP32 family otherwise; register precisions (A, B as in memory, C FP32).
+  public init(descriptor: GEMMDescriptor) {
+    var d = descriptor.c
+    check(mfa_gemm_descriptor_kernel_descriptor(&d, &c))
+  }
+
+  public var blockDimensions: (M: UInt16, N: UInt16, K: UInt16)? {
+    get { c.has_block_dimensions != 0 ? c.block_dimensions : nil }
+    set {
+      c.has_block_dimensions = newValue == nil ? 0 : 1
+      if let v = newValue { c.block_dimensions = (v.M, v.N, v.K) }
+    }
+  }
+  public var leadingBlockDimensions: (A: UInt16, B: UInt16, C: UInt16)? {
+    get { c.has_leading_block_dimensions != 0 ? c.leading_block_dimensions : nil }
+    set {
+      c.has_leading_block_dimensions = newValue == nil ? 0 : 1
+      if let v = newValue { c.leading_block_dimensions = (v.A, v.B, v.C) }
+    }
+  }
+  private static func precisions(_ t: (UInt8, UInt8, UInt8))
+    -> (A: GEMMOperandPrecision, B: GEMMOperandPrecision, C: GEMMOperandPrecision) {
+    (GEMMOperandPrecision(rawValue: UInt16(t.0))!, GEMMOperandPrecision(rawValue: UInt16(t.1))!,
+     GEMMOperandPrecision(rawValue: UInt16(t.2))!)
+  }
+  public var memoryPrecisions: (A: GEMMOperandPrecision, B: GEMMOperandPrecision, C: GEMMOperandPrecision)? {
+    get { c.has_memory_precisions != 0 ? Self.precisions(c.memory_precisions) : nil }
+    set {
+      c.has_memory_precisions = newValue == nil ? 0 : 1
+      if let v = newValue { c.memory_precisions = (UInt8(v.A.rawValue), UInt8(v.B.rawValue), UInt8(v.C.rawValue)) }
+    }
+  }
+  public var registerPrecisions: (A: GEMMOperandPrecision, B: GEMMOperandPrecision, C: GEMMOperandPrecision)? {
+    get { c.has_register_precisions != 0 ? Self.precisions(c.register_precisions) : nil }
+    set {
+      c.has_register_precisions = newValue == nil ? 0 : 1
+      if let v = newValue { c.register_precisions = (UInt8(v.A.rawValue), UInt8(v.B.rawValue), UInt8(v.C.rawValue)) }
+    }
+  }
+  public var preferAsyncLoad: Bool {
+    get { c.prefer_async_load != 0 }
+    set { c.prefer_async_load = newValue ? 1 : 0 }
+  }
+  public var preferAsyncStore: Bool? {
+    get { c.prefer_async_store == 0xFF ? nil : c.prefer_async_store != 0 }
+    set { c.prefer_async_store = newValue.map { $0 ? 1 : 0 } ?? 0xFF }
+  }
+  public var splits: (M: UInt16, N: UInt16)? {
+    get { c.has_splits != 0 ? c.splits : nil }
+    set {
+      c.has_splits = newValue == nil ? 0 : 1
+      if let v = newValue { c.splits = (v.M, v.N) }
+    }
+  }
+  public var transposeState: (A: Bool, B: Bool)? {
+    get { c.has_transpose_state != 0 ? (c.transpose_A != 0, c.transpose_B != 0) : nil }
+    set {
+      c.has_transpose_state = newValue == nil ? 0 : 1
+      if let v = newValue { c.transpose_A = v.A ? 1 : 0; c.transpose_B = v.B ? 1 : 0 }
+    }
+  }
+  /// B200 extension: which sm_100a kernel family the heuristic picked.
+  public var backend: AttentionBackend {
+    get { AttentionBackend(rawValue: c.backend)! }
+    set { c.backend = newValue.rawValue }
+  }
+}
+
+/// GEMMKernel.swift:10-270
+public final class GEMMKernel {
+  let handle: OpaquePointer
+  let owned: Bool
+
+  public init(descriptor: GEMMKernelDescriptor) {
+    var kd = descriptor.c
+    var out: OpaquePointer?
+    check(mfa_gemm_kernel_create(&kd, &out))
+    handle = out!
+    owned = true
+  }
+  init(cached descriptor: GEMMDescriptor) {
+    var d = descriptor.c
+    var out: OpaquePointer?
+    check(mfa_gemm_kernel_cache_fetch(&d, &out))
+    handle = out!
+    owned = false
+  }
+  deinit { if owned { mfa_gemm_kernel_destroy(handle) } }
+
+  /// GEMMDescriptor+PipelineCache.swift:24-36: creates the descriptor's kernel object once.  The cache key is the
+  /// precisions and transposes; M, N, K, leading dimensions, loadPreviousC and the batch are launch constants.
+  public static func register(descriptor: GEMMDescriptor) { _ = GEMMKernel(cached: descriptor) }
+  /// `pipelineCache[descriptor]`: the library-owned kernel object (registered on first use).
+  public static func cached(descriptor: GEMMDescriptor) -> GEMMKernel { GEMMKernel(cached: descriptor) }
+  public static var cacheSize: Int { Int(mfa_gemm_kernel_cache_size()) }
+
+  public var blockDimensions: (M: UInt16, N: UInt16, K: UInt16) {
+    var out: (UInt16, UInt16, UInt16) = (0, 0, 0)
+    withUnsafeMutablePointer(to: &out) {
+      $0.withMemoryRebound(to: UInt16.self, capacity: 3) { check(mfa_gemm_kernel_block_dimensions(handle, $0)) }
+    }
+    return out
+  }
+  public var threadgroupSize: UInt32 {
+    var out: UInt32 = 0
+    check(mfa_gemm_kernel_threadgroup_size(handle, &out))
+    return out
+  }
+  public var threadgroupMemoryAllocation: UInt32 {
+    var out: UInt32 = 0
+    check(mfa_gemm_kernel_threadgroup_memory_allocation(handle, &out))
+    return out
+  }
+  /// Output tiles: ceil(N / block N) * ceil(M / block M) * batch (AdversarialShapeTest.swift:155-158).
+  public func gridSize(constants: mfa_gemm_function_constants_t) -> UInt32 {
+    var constants = constants
+    var out: UInt32 = 0
+    check(mfa_gemm_kernel_grid_size(handle, &constants, &out))
+    return out
+  }
+  /// CUDA kernels one `encode` launches: 1, plus a staging copy per 16-bit operand TMA cannot address in place.
+  public func launchCount(constants: mfa_gemm_function_constants_t) -> UInt32 {
+    var constants = constants
+    var out: UInt32 = 0
+    check(mfa_gemm_kernel_launch_count(handle, &constants, &out))
+    return out
+  }
+  /// Stands in for `createSource()`: the name of the ahead-of-time compiled kernel.
+  public var sourceName: String { String(cString: mfa_gemm_kernel_source_name(handle)) }
+
+  /// Binds A, B, C (DEVICE pointers, bindings 0, 1, 2 as in GEMMKernel+Source.swift:42-44) and dispatches on `stream`
+  /// (a cudaStream_t): what AdversarialShapeTest.swift:140-169 does by hand around the Metal pipeline.
+  public func encode(constants: mfa_gemm_function_constants_t,
+                     A: UnsafeRawPointer, B: UnsafeRawPointer, C: UnsafeMutableRawPointer,
+                     stream: UnsafeMutableRawPointer? = nil) {
+    var table: [UnsafeMutableRawPointer?] = [UnsafeMutableRawPointer(mutating: A), UnsafeMutableRawPointer(mutating: B), C]
+    var constants = constants
+    check(mfa_gemm_kernel_encode(handle, &constants, &table, stream))
   }
 }
